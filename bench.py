@@ -53,7 +53,16 @@ def parse():
     ap.add_argument("--no-gpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the config-2 (TG) block of the N = 1 line")
     ap.add_argument("--profile-out", default=None, help="write the per-kernel-family event profile to this JSON file")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last of them returned, its loss, as DIR/loss.npy "
+                         "(float32); the inputs are seeded, so two builds run with the same arguments can be compared "
+                         "output for output")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return a
 
 
 def load_traffic(workload, batch):
@@ -88,11 +97,14 @@ def load_peaks():
 # ---------------------------------------------------------------------------
 def run_cpu_port(workload, steps, warmup, budget_s):
     """The reference's CPU path on the host cores, in a CUDA-free subprocess: the UNMODIFIED reference modules when they
-    are available (/root/reference, or the copies oracle/build.py staged under oracle/_ref/ -- kind "reference"), else
-    the oracle port (kind "port")."""
+    are available (the checkout oracle/ref_shim.py finds, or the copies oracle/build.py staged under oracle/_ref/ -- kind
+    "reference"), else the oracle port (kind "port"), said on stderr."""
     from oracle import ref_shim
     use_ref = ref_shim.available() or ref_shim.staged_available()
     mod = "oracle.ref_baseline" if use_ref else "oracle.cpu_baseline"
+    if not use_ref:
+        print("bench: no upstream uoo723/PMGT reference (set PMGT_REFERENCE_ROOT, or stage it with build()); the CPU "
+              "arm times the oracle port (kind \"port\")", file=sys.stderr)
     cmd = [sys.executable, "-m", mod, "--workload", workload, "--steps", str(steps), "--warmup", str(warmup),
            "--budget-s", str(budget_s)]
     env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
@@ -100,6 +112,8 @@ def run_cpu_port(workload, steps, warmup, budget_s):
         env.pop(k, None)
     r = subprocess.run(cmd, cwd=ROOT, env=env, capture_output=True, text=True, timeout=1500)
     if r.returncode != 0 and use_ref:  # never lose the line over the staged copy: fall back to the port, and say so
+        print("bench: the reference's own modules failed; the CPU arm times the oracle port (kind \"port\"):\n"
+              + r.stderr[-1000:], file=sys.stderr)
         cmd[2] = "oracle.cpu_baseline"
         r = subprocess.run(cmd, cwd=ROOT, env=env, capture_output=True, text=True, timeout=1500)
     if r.returncode != 0:
@@ -134,8 +148,8 @@ def reference_arm(a):
               f"the {wl} graph; {how}; {d['cores']} cores")
     line = {
         "impl": "reference", "metric": "pmgt_pretrain_node_contexts_per_s", "value": d["value"], "unit": "contexts/s",
-        "n_gpus": a.gpus, "steps": a.steps, "warmup": a.warmup, "ms_per_step": d["ms_per_step"], "higher_is_better": True,
-        "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
+        "n_gpus": a.gpus, "steps": d["steps"], "warmup": d["warmup"], "ms_per_step": d["ms_per_step"],
+        "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": workload_config(wl, d["targets_per_step"], "cpu"),
         "cpu_baseline": {"value": d["value"], "unit": "contexts/s", "cores": d["cores"], "kind": d["kind"], "sample": sample,
                          "sampler_contexts_per_s": d["sampler_contexts_per_s"], "model_contexts_per_s": d["model_contexts_per_s"]},
@@ -258,9 +272,12 @@ def k3_flops_per_step(cfg_over, batch, L):
     return 3.0 * per_seq_layer * layers * 12 * batch
 
 
-def measure(a, workload, steps, warmup, profile, rank, local_rank, ws, dev):
+def measure(a, workload, steps, warmup, profile, rank, local_rank, ws, dev, dump_dir=None):
     """Builds the workload, runs the device-resident series (`value`), the end-to-end series (`e2e`) and, if asked,
-    the per-kernel-family event profile.  Returns a dict of results (rank 0 carries the roofline)."""
+    the per-kernel-family event profile.  Returns a dict of results (rank 0 carries the roofline).  With `dump_dir`,
+    rank 0 writes there what the last step of the device-resident series returned, its loss.  The parameters and
+    gradients that step leaves are not written: the backward pass sums gradients with floating-point atomics and AdamW
+    amplifies the rounding differences, so after a few steps they differ from run to run by far more than rounding."""
     import numpy as np
     import torch
     import torch.distributed as dist
@@ -326,12 +343,15 @@ def measure(a, workload, steps, warmup, profile, rank, local_rank, ws, dev):
     launches0 = ops.LAUNCHES[0]
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    run_steps(idx_dev, warmup, steps)
+    last_loss = run_steps(idx_dev, warmup, steps)
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
     launches = ops.LAUNCHES[0] - launches0
     clk = clocks.stop() if rank == 0 else None
+    if dump_dir and rank == 0:
+        os.makedirs(dump_dir, exist_ok=True)
+        np.save(os.path.join(dump_dir, "loss.npy"), last_loss.float().cpu().numpy())
     t = torch.tensor([ms], device=dev)
     if ws > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -479,7 +499,7 @@ def ours(a):
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     dev = torch.device("cuda", local_rank)
 
-    main_res = measure(a, a.workload, a.steps, a.warmup, True, rank, local_rank, ws, dev)
+    main_res = measure(a, a.workload, a.steps, a.warmup, True, rank, local_rank, ws, dev, dump_dir=a.dump_outputs)
     if rank == 0 and a.profile_out and main_res["profile"]:
         with open(a.profile_out, "w") as f:
             json.dump(main_res["profile"], f, indent=1)

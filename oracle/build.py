@@ -3,11 +3,12 @@
 ``build()``      the CPU replay of the Philox sampler stream -> ``oracle/_build/liboracle.so``.
 ``build_ref()``  the reference is pure Python, so "building" it means staging the UNMODIFIED hot-path modules
                  (pmgt/pmgt/{datasets,models,modeling_pmgt,configuration_pmgt,utils}.py, pmgt/optimizers.py and the
-                 two package __init__ files) from ``/root/reference`` into the git-ignored ``oracle/_ref/``.  That
-                 directory is build output: it never enters the history, but it travels to the GPU box with the
-                 snapshot, where ``bench.py --impl reference`` and the ``cpu_baseline`` leg then time the reference's OWN
-                 sampler and model code on the host cores (``kind: "reference"``) instead of the oracle port.  Runs only
-                 where ``/root/reference`` exists (this container); elsewhere the staged copy is used as is.
+                 two package __init__ files) from the upstream checkout ``ref_shim`` finds (``PMGT_REFERENCE_ROOT``, or
+                 an importable ``pmgt`` package) into the git-ignored ``oracle/_ref/``.  That directory is build output:
+                 it never enters the history, but a copy of the tree that carries it lets ``bench.py --impl reference``
+                 and the ``cpu_baseline`` leg time the reference's OWN sampler and model code on the host cores
+                 (``kind: "reference"``) instead of the oracle port.  Without a checkout an existing staged copy is used
+                 as is.
 """
 import ctypes
 import os
@@ -26,7 +27,6 @@ def build(force: bool = False) -> str:
     return OUT
 
 
-REF_ROOT = os.environ.get("PMGT_REFERENCE_ROOT", "/root/reference")
 REF_OUT = os.path.join(HERE, "_ref")
 REF_FILES = ["pmgt/__init__.py", "pmgt/optimizers.py", "pmgt/pmgt/__init__.py", "pmgt/pmgt/datasets.py",
              "pmgt/pmgt/models.py", "pmgt/pmgt/modeling_pmgt.py", "pmgt/pmgt/configuration_pmgt.py", "pmgt/pmgt/utils.py"]
@@ -37,7 +37,9 @@ def build_ref(force: bool = False) -> str:
     "" when neither the reference tree nor a staged copy is available."""
     import shutil
 
-    if os.path.isdir(os.path.join(REF_ROOT, "pmgt", "pmgt")):
+    from oracle.ref_shim import REFERENCE_ROOT as REF_ROOT
+
+    if REF_ROOT and os.path.isdir(os.path.join(REF_ROOT, "pmgt", "pmgt")):
         for rel in REF_FILES:
             src, dst = os.path.join(REF_ROOT, rel), os.path.join(REF_OUT, rel)
             os.makedirs(os.path.dirname(dst), exist_ok=True)

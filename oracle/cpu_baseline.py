@@ -9,7 +9,7 @@ Runs the oracle *port* of the reference's pre-training step on the host cores:
            fp32, torch.set_num_threads(all cores), with the reference's per-target
            pair-encoding loop replaced by one batched call (an *optimistic* baseline:
            the batched call is ~4.9x faster than the loop on CPU, SURVEY section 6).
-/root/reference itself cannot travel to the GPU box, hence kind = "port".
+The upstream reference is not part of this repository, hence kind = "port".
 Only bench.py may call this (cpu_baseline leg and --impl reference).
 """
 import multiprocessing as mp

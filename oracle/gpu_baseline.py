@@ -1,7 +1,7 @@
 """TEST / BENCH INFRASTRUCTURE ONLY -- the reference's model step run EAGERLY on the GPU (BASELINE.md section 4 item 5,
 SURVEY section 2.2: "the bar is beat stock PyTorch eager on the same B200").
 
-The unmodified reference cannot travel to the GPU box (``/root/reference`` is absent there), so this is the oracle
+The unmodified reference is not part of this repository, so this is the oracle
 restatement (``oracle/model_ref.py``, pinned to the reference by the golden vectors) executed the way the reference
 executes it (``pmgt/pmgt/models.py:56-176``): fp32 stock PyTorch ops on ``cuda:0``, feature rows gathered with
 ``nn.Embedding``-style indexing, ONE encoder call for the targets, then the reference's Python loop over targets with a

@@ -4,12 +4,12 @@ A functional (no ``nn.Module``) restatement of the reference's pre-training
 forward pass, operating on a plain ``dict`` of tensors that uses the
 reference's state-dict key names.  Autograd provides the gradients.  Pinned in
 ``tests/test_oracle_model.py`` against the unmodified reference (when
-``/root/reference`` is present) and against the committed golden vectors in
+``PMGT_REFERENCE_ROOT`` names a checkout) and against the committed golden vectors in
 ``tests/golden/model_golden.pt`` (generated from the unmodified reference by
 ``tests/golden/make_golden.py``).
 
 Third-party arithmetic restated here (transformers==4.11.2, absent from
-/root/reference): BertSelfOutput / BertOutput = dense -> dropout ->
+the reference tree): BertSelfOutput / BertOutput = dense -> dropout ->
 LayerNorm(x + residual); BertIntermediate = dense -> erf-GELU;
 get_extended_attention_mask = (1 - mask)[:, None, None, :] * -10000.
 """

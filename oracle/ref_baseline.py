@@ -1,6 +1,6 @@
 """TEST / BENCH INFRASTRUCTURE ONLY -- the UNMODIFIED reference's pre-training path timed on the host CPU cores.
 
-Uses the reference's own modules (``/root/reference`` in the build container, else the byte-for-byte copies
+Uses the reference's own modules (the checkout named by ``PMGT_REFERENCE_ROOT``, else the byte-for-byte copies
 ``oracle/build.py::build_ref`` staged under the git-ignored ``oracle/_ref/``) through ``oracle/ref_shim.py`` (transformers
 5.x -> 4.11.2 semantics, no edits to the reference code):
 
@@ -122,7 +122,7 @@ def run_cli(argv=None):
         "targets_per_step": B, "cores": cores, "value": ctx / (t_sample_timed + t_model),
         "sampler_contexts_per_s": ctx / t_sample_timed, "model_contexts_per_s": ctx / t_model, "loss_last": loss,
         "ms_per_step": 1e3 * (t_sample_timed + t_model) / a.steps, "kind": "reference",
-        "reference_root": "/root/reference" if from_tree else "oracle/_ref (staged copy of the unmodified modules)",
+        "reference_root": ref_shim.REFERENCE_ROOT if from_tree else "oracle/_ref (staged copy of the unmodified modules)",
     }))
 
 

@@ -1,10 +1,10 @@
 """TEST INFRASTRUCTURE ONLY -- import shim for the *unmodified* reference.
 
-Makes ``/root/reference`` (uoo723/PMGT, pinned to transformers 4.11.2) importable
-under the transformers 5.x that ships in this image, without editing the
-reference tree.  Only usable inside the build container (the GPU box has no
-``/root/reference``); it is used by ``tests/golden/make_golden.py`` to generate
-the committed golden vectors and by CPU-side tests that cross-check
+Makes a checkout of the upstream reference (uoo723/PMGT, pinned to
+transformers 4.11.2) importable under transformers 5.x, without editing the
+reference tree.  The checkout is not part of this repository: it is used when
+``PMGT_REFERENCE_ROOT`` names it or its ``pmgt`` package is importable, by ``tests/golden/make_golden.py`` to
+generate the committed golden vectors and by CPU-side tests that cross-check
 ``oracle/model_ref.py`` / ``oracle/sampler_ref.py`` against the real thing.
 
 Nothing under ``pmgt_b200/`` may import this module.
@@ -12,22 +12,40 @@ Nothing under ``pmgt_b200/`` may import this module.
 import os
 import sys
 
-REFERENCE_ROOT = os.environ.get("PMGT_REFERENCE_ROOT", "/root/reference")
+def _find_root() -> str:
+    """``PMGT_REFERENCE_ROOT``, else the checkout whose upstream ``pmgt`` package is importable (installed, or its root
+    on ``sys.path``); "" when there is neither."""
+    root = os.environ.get("PMGT_REFERENCE_ROOT")
+    if root:
+        return root
+    import importlib.util
+
+    try:
+        spec = importlib.util.find_spec("pmgt")
+    except (ImportError, ValueError):
+        return ""
+    for loc in (spec.submodule_search_locations or []) if spec else []:
+        if os.path.isdir(os.path.join(loc, "pmgt")):
+            return os.path.dirname(os.path.abspath(loc))
+    return ""
+
+
+REFERENCE_ROOT = _find_root()
 STAGED_ROOT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")   # oracle/build.py::build_ref()
 
 
 def available() -> bool:
-    """The reference tree itself (build container only): what the parity tests and the golden generator need."""
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, "pmgt", "pmgt"))
+    """The reference tree itself (``_find_root``): what the parity tests and the golden generator need."""
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, "pmgt", "pmgt"))
 
 
 def staged_available() -> bool:
-    """The unmodified hot-path modules staged under oracle/_ref/ (travels to the GPU box; bench CPU arm only)."""
+    """The unmodified hot-path modules staged under oracle/_ref/ (bench CPU arm only)."""
     return os.path.isdir(os.path.join(STAGED_ROOT, "pmgt", "pmgt"))
 
 
 def load_any():
-    """The reference from /root/reference when present, else from the staged copy."""
+    """The reference tree when present, else the staged copy."""
     global REFERENCE_ROOT
     if not available() and staged_available():
         REFERENCE_ROOT = STAGED_ROOT
@@ -44,7 +62,8 @@ def load(_root_ok: bool = False):
     if _loaded is not None:
         return _loaded
     if not _root_ok and not available():
-        raise RuntimeError(f"reference tree not present at {REFERENCE_ROOT}")
+        raise RuntimeError(f"no reference tree at {REFERENCE_ROOT!r}: set PMGT_REFERENCE_ROOT to a checkout of "
+                           "uoo723/PMGT")
     sys.dont_write_bytecode = True  # the reference tree is read-only
     if REFERENCE_ROOT not in sys.path:
         sys.path.insert(0, REFERENCE_ROOT)

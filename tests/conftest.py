@@ -13,7 +13,7 @@ warnings.filterwarnings("ignore", message=".*use_return_dict.*")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: test needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "needs_reference: test imports /root/reference (build container only)")
+    config.addinivalue_line("markers", "needs_reference: test imports a checkout of the upstream uoo723/PMGT (oracle/ref_shim.py)")
 
 
 def _has_cuda():
@@ -32,7 +32,7 @@ def pytest_collection_modifyitems(config, items):
     have_cuda = _has_cuda()
     for item in items:
         if "needs_reference" in item.keywords and not have_ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present on this box"))
+            item.add_marker(pytest.mark.skip(reason="no checkout of uoo723/PMGT found: set PMGT_REFERENCE_ROOT"))
         if "gpu" in item.keywords and not have_cuda:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
 

@@ -1,8 +1,8 @@
 """Generates the committed golden vectors from the UNMODIFIED reference.
 
-Run in the build container only (needs /root/reference):
+Needs a checkout of the upstream reference (uoo723/PMGT):
 
-    python tests/golden/make_golden.py
+    PMGT_REFERENCE_ROOT=<checkout> python tests/golden/make_golden.py
 
 Outputs (small, committed):
   tests/golden/model_golden.pt        reference PMGT.forward/backward outputs for two

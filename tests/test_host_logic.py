@@ -24,6 +24,32 @@ def test_state_dict_keys_match_reference_golden(golden_dir):
     assert not any(p.requires_grad for p in net.feat_embeddings.parameters())
 
 
+@pytest.mark.parametrize("name", ["default", "multihead"])
+def test_state_dict_layout_and_roundtrip_match_reference_golden(golden_dir, name):
+    """The reference's state-dict layout as tests/golden/make_golden.py certified it: the reference loaded
+    model_ref.init_state_dict(cfg) with strict=False (any shape mismatch raises) with no unexpected key and only the
+    position_ids / role_ids buffers missing, and its named_parameters() order is the key order of grad_norms."""
+    from oracle import model_ref
+    g = torch.load(os.path.join(golden_dir, "model_golden.pt"), weights_only=False)[name]
+    cfg = g["cfg"]
+    ref_sd = model_ref.init_state_dict(cfg, g["node_size"], seed=g["weights_seed"], perturb=g["weights_perturb"])
+    config = PMGTConfig(hidden_size=cfg["hidden_size"], feat_hidden_sizes=cfg["feat_hidden_sizes"],
+                        num_hidden_layers=cfg["num_hidden_layers"], num_attention_heads=cfg["num_attention_heads"],
+                        intermediate_size=cfg["intermediate_size"], beta=cfg["beta"])
+    ours = PMGT(g["node_size"], cfg["random_node_ratio"], cfg["mask_node_ratio"], config,
+                feat_init_emb=[ref_sd[f"feat_embeddings.{m}.weight"].numpy() for m in range(2)])
+    assert [n for n, p in ours.named_parameters() if p.requires_grad] == list(g["grad_norms"])
+    sd = ours.state_dict()
+    assert set(sd) == set(ref_sd) | {"bert.embeddings.position_ids", "bert.embeddings.role_ids"}
+    for k, v in ref_sd.items():
+        assert sd[k].shape == v.shape and sd[k].dtype == v.dtype, (k, sd[k].shape, sd[k].dtype, v.shape, v.dtype)
+    missing, unexpected = ours.load_state_dict(ref_sd, strict=False)   # reference checkpoint -> ours
+    assert not unexpected and sorted(missing) == ["bert.embeddings.position_ids", "bert.embeddings.role_ids"]
+    back = ours.state_dict()                                            # and back out, unchanged
+    for k, v in ref_sd.items():
+        assert torch.equal(back[k], v), k
+
+
 @pytest.mark.needs_reference
 def test_state_dict_roundtrip_with_live_reference():
     from oracle import ref_shim
@@ -184,6 +210,20 @@ def test_bench_batch_resolution_weak_and_strong():
         bench.resolve_batch(4096, 8190, 4)
     with pytest.raises(SystemExit):
         bench.resolve_batch(4096, 4, 8)
+
+
+def test_bench_argument_checks(tmp_path, monkeypatch):
+    """bench.py: --steps is the number of timed steps and must be at least 1; --dump-outputs belongs to --impl ours."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(os.path.dirname(os.path.dirname(__file__)), "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    monkeypatch.setattr("sys.argv", ["bench.py", "--steps", "7", "--dump-outputs", str(tmp_path)])
+    assert bench.parse().steps == 7
+    for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        monkeypatch.setattr("sys.argv", ["bench.py", *argv])
+        with pytest.raises(SystemExit):
+            bench.parse()
 
 
 @pytest.mark.parametrize("n,batch,ws", [(1000, 128, 1), (1000, 128, 4), (130, 64, 8), (64, 64, 2), (10, 64, 4)])

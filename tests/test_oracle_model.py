@@ -1,6 +1,6 @@
 """Pins oracle/model_ref.py (the fp32 torch restatement) against the golden
-vectors generated from the unmodified reference, and -- when /root/reference is
-present -- against the reference itself on fresh inputs."""
+vectors generated from the unmodified reference, and -- when PMGT_REFERENCE_ROOT
+names a checkout of it -- against the reference itself on fresh inputs."""
 import os
 
 import pytest
@@ -61,6 +61,20 @@ def test_mask_nodes_follows_reference_rng_order(golden_dir):
     assert torch.equal(ids, g["masked_ids"]) and torch.equal(m, g["masked_mask"]) and torch.equal(tgt, g["masked_target_idx"])
 
 
+@pytest.mark.parametrize("name", ["default", "multihead"])
+def test_oracle_masking_inside_forward_matches_reference_golden(golden_dir, name):
+    """The reference drew its NFR corruption inside PMGT.forward under torch.manual_seed(torch_seed); the oracle, left
+    to draw it itself under the same seed, reproduces the stored loss and logits."""
+    g = _load(golden_dir, name)
+    sd = model_ref.init_state_dict(g["cfg"], g["node_size"], seed=g["weights_seed"], perturb=g["weights_perturb"])
+    torch.manual_seed(g["torch_seed"])
+    with torch.no_grad():
+        out = model_ref.pretrain_forward(sd, g["cfg"], g["node_size"], g["target"], g["pair"], g["num_pairs"],
+                                         g["labels"], training=True)
+    assert torch.allclose(out["loss"], g["loss"], rtol=1e-5, atol=1e-6)
+    assert torch.allclose(out["prediction_logits"], g["prediction_logits"], rtol=1e-4, atol=1e-5)
+
+
 def test_adamw_oracle_matches_reference_golden(golden_dir):
     g = torch.load(os.path.join(golden_dir, "adamw_golden.pt"), weights_only=False)
     p = g["p0"].clone()
@@ -73,7 +87,7 @@ def test_adamw_oracle_matches_reference_golden(golden_dir):
 
 @pytest.mark.needs_reference
 def test_oracle_matches_live_reference():
-    """Fresh inputs, live reference (build container only)."""
+    """Fresh inputs, live reference (PMGT_REFERENCE_ROOT)."""
     R = ref_shim.load()
     cfg = model_ref.default_cfg(num_hidden_layers=2, mask_node_ratio=0.5)
     node_size = 30

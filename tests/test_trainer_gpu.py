@@ -169,3 +169,33 @@ def test_gradient_accumulation_and_rejected_flags(tmp_path):
     assert float((g2 - g1).abs().max()) > 0 and float(g2.norm()) > 0.5 * float(g1.norm())   # accumulated, not replaced
     tm.train_on_indices(ds, np.arange(128, 192), 0)
     assert tm.global_step == 1                                      # gradients were reset, a new cycle started
+
+
+def test_bench_times_exactly_steps_and_dumps_the_last_timed_loss(tmp_path, monkeypatch):
+    """bench.py: after --warmup steps the device-resident series runs exactly --steps steps, and --dump-outputs writes
+    the loss the last of them returned (float32 DIR/loss.npy)."""
+    import importlib.util
+    from pmgt_b200 import trainer
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(os.path.dirname(os.path.dirname(__file__)), "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    dump = tmp_path / "dump"
+    monkeypatch.setattr("sys.argv", ["bench.py", "--workload", "VG", "--batch", "64", "--steps", "3", "--warmup", "2",
+                                     "--dump-outputs", str(dump)])
+    a = bench.parse()
+    calls = []
+    step = trainer.PMGTTrainerModel.train_on_indices
+
+    def counted(self, dataset, indices, epoch):
+        loss = step(self, dataset, indices, epoch)
+        calls.append((epoch, float(loss)))
+        return loss
+
+    monkeypatch.setattr(trainer.PMGTTrainerModel, "train_on_indices", counted)
+    bench.measure(a, a.workload, a.steps, a.warmup, False, 0, 0, 1, torch.device("cuda", 0), dump_dir=a.dump_outputs)
+    total = a.warmup + a.steps
+    # warmup, the timed device-resident series, then the end-to-end series (as many steps again)
+    assert [e for e, _ in calls] == list(range(total)) + list(range(total, total + a.steps))
+    got = np.load(dump / "loss.npy")
+    assert got.dtype == np.float32 and np.isfinite(got)
+    assert float(got) == calls[total - 1][1]
