@@ -39,7 +39,7 @@ typedef enum pmgt_status {
 } pmgt_status;
 
 /* ABI version of this header; bumped on any signature change. */
-#define PMGT_B200_ABI_VERSION 12
+#define PMGT_B200_ABI_VERSION 13
 int pmgt_abi_version(void);
 const char* pmgt_last_error(void);
 
@@ -231,6 +231,39 @@ typedef struct pmgt_embed_args {
 
 int pmgt_embed_fuse_fwd(const pmgt_embed_args* a, void* stream);
 int pmgt_embed_fuse_bwd(const pmgt_embed_args* a, void* stream);
+
+/*
+ * The same fusion for any number of feature modalities M = n_mod in [1, PMGT_MAX_MODALITIES] (the reference's
+ * PMGTEmbeddings takes one feat_linear per entry of feat_hidden_sizes and a Linear(M*H -> M) modality attention):
+ * pmgt_embed_args with every per-modality pair turned into an array indexed by modality.
+ *   e[m]        [T][H] (or [table_rows][H] with row_idx) bf16 projected features of modality m
+ *   w_att [M][M*H], b_att [M] fp32; d_w_att / d_b_att the same shapes
+ *   de[m]       bwd: [T][H] bf16 gradient of e[m];  de_acc[m]: projected-table mode, [table_rows][H] fp32, red.add
+ *   d_bias[m]   bwd: [H] fp32 column sums of de[m], accumulated
+ * Entries m >= n_mod are ignored.  n_mod == 2 runs pmgt_embed_fuse_fwd / _bwd with the equivalent pmgt_embed_args.
+ * Otherwise H is a multiple of 8 in [8, 1024] and every matrix is 16-byte aligned.  The dropout mask is the one of
+ * pmgt_embed_fuse_fwd (element tok * H + h under dropout_seed / dropout_site), whatever M is.  At n_mod == 1 the
+ * softmax weight is exactly 1 and d_w_att / d_b_att receive exact zeros.
+ */
+#define PMGT_MAX_MODALITIES 4
+
+typedef struct pmgt_embed_multi_args {
+  int64_t rows; int L; int H; int n_mod;
+  const uint16_t* e[PMGT_MAX_MODALITIES];
+  const float* w_att; const float* b_att; const float* pos; const float* role;
+  const float* ln_g; const float* ln_b; float ln_eps;
+  float dropout_p; uint64_t dropout_seed; uint32_t dropout_site;
+  uint16_t* x_out;            /* fwd */
+  const uint16_t* dx;         /* bwd: [T][H] bf16 */
+  uint16_t* de[PMGT_MAX_MODALITIES];
+  float* d_w_att; float* d_b_att; float* d_pos; float* d_role; float* d_ln_g; float* d_ln_b;
+  float* d_bias[PMGT_MAX_MODALITIES];
+  const uint16_t* dx_b;       /* bwd, optional: second gradient term, summed with dx */
+  const int64_t* row_idx; float* de_acc[PMGT_MAX_MODALITIES]; int skip_row0;
+} pmgt_embed_multi_args;
+
+int pmgt_embed_multi_fwd(const pmgt_embed_multi_args* a, void* stream);
+int pmgt_embed_multi_bwd(const pmgt_embed_multi_args* a, void* stream);
 
 /*
  * Gather-fused feature projection for large graphs, H = 128 (csrc/gather_proj.cu): persistent tcgen05 kernels whose

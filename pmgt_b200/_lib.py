@@ -11,7 +11,7 @@ import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libpmgt_b200.so")
-ABI_VERSION = 12
+ABI_VERSION = 13
 
 _lib = None
 
@@ -57,6 +57,28 @@ class EmbedArgs(C.Structure):
         ("d_bias_v", c_vp), ("d_bias_t", c_vp),
         ("dx_b", c_vp),
         ("row_idx", c_vp), ("dev_acc", c_vp), ("det_acc", c_vp), ("skip_row0", C.c_int),
+    ]
+
+
+MAX_MODALITIES = 4  # PMGT_MAX_MODALITIES
+_PerMod = c_vp * MAX_MODALITIES
+
+
+class EmbedMultiArgs(C.Structure):
+    _fields_ = [
+        ("rows", C.c_int64), ("L", C.c_int), ("H", C.c_int), ("n_mod", C.c_int),
+        ("e", _PerMod),
+        ("w_att", c_vp), ("b_att", c_vp), ("pos", c_vp), ("role", c_vp),
+        ("ln_g", c_vp), ("ln_b", c_vp), ("ln_eps", C.c_float),
+        ("dropout_p", C.c_float), ("dropout_seed", C.c_uint64), ("dropout_site", C.c_uint32),
+        ("x_out", c_vp),
+        ("dx", c_vp),
+        ("de", _PerMod),
+        ("d_w_att", c_vp), ("d_b_att", c_vp), ("d_pos", c_vp), ("d_role", c_vp),
+        ("d_ln_g", c_vp), ("d_ln_b", c_vp),
+        ("d_bias", _PerMod),
+        ("dx_b", c_vp),
+        ("row_idx", c_vp), ("de_acc", _PerMod), ("skip_row0", C.c_int),
     ]
 
 
@@ -203,6 +225,8 @@ SIGNATURES = {
     "pmgt_gather_proj_dw": (C.c_int, [C.POINTER(GatherProjArgs), c_vp]),
     "pmgt_embed_fuse_fwd": (C.c_int, [C.POINTER(EmbedArgs), c_vp]),
     "pmgt_embed_fuse_bwd": (C.c_int, [C.POINTER(EmbedArgs), c_vp]),
+    "pmgt_embed_multi_fwd": (C.c_int, [C.POINTER(EmbedMultiArgs), c_vp]),
+    "pmgt_embed_multi_bwd": (C.c_int, [C.POINTER(EmbedMultiArgs), c_vp]),
     "pmgt_attn_core_fwd": (C.c_int, [C.POINTER(AttnArgs), c_vp]),
     "pmgt_attn_core_bwd": (C.c_int, [C.POINTER(AttnArgs), c_vp]),
     "pmgt_res_ln_fwd": (C.c_int, [C.POINTER(ResLnArgs), c_vp]),

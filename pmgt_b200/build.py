@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ_DIR = os.path.join(HERE, "csrc", "_obj")
 OUT = os.path.join(HERE, "libpmgt_b200.so")
-SOURCES = ["api.cu", "sampler.cu", "graph_build.cu", "gemm_umma.cu", "gather_proj.cu", "linear_tile.cu", "ffn_block.cu", "rowwise.cu", "res_ln_wide.cu", "embed128.cu", "ln_bwd_stream.cu", "attention.cu", "attention_small.cu", "attention_mma.cu", "attention_mid.cu", "attention_reg.cu", "loss.cu", "peer_reduce.cu"]
+SOURCES = ["api.cu", "sampler.cu", "graph_build.cu", "gemm_umma.cu", "gather_proj.cu", "linear_tile.cu", "ffn_block.cu", "rowwise.cu", "res_ln_wide.cu", "embed128.cu", "embed_multi.cu", "ln_bwd_stream.cu", "attention.cu", "attention_small.cu", "attention_mma.cu", "attention_mid.cu", "attention_reg.cu", "loss.cu", "peer_reduce.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

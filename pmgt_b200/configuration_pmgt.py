@@ -8,6 +8,9 @@ keeps the attributes the reference's model code reads from that base class:
 import copy
 import json
 
+# PMGT_MAX_MODALITIES of include/pmgt_b200.h: the embedding fusion kernels take one to four feature modalities
+MAX_MODALITIES = 4
+
 
 class PMGTConfig:
     model_type = "pmgt"
@@ -58,8 +61,9 @@ class PMGTConfig:
             raise ValueError("pmgt_b200 implements the reference's only activation, erf-GELU (hidden_act='gelu')")
         if getattr(self, "position_embedding_type", "absolute") != "absolute":
             raise ValueError("only absolute position embeddings are supported (the reference never enables the others)")
-        if len(self.feat_hidden_sizes) != 2:
-            raise ValueError("pmgt_b200 supports exactly two modalities (visual, textual) like the reference's data")
+        if not 1 <= len(self.feat_hidden_sizes) <= MAX_MODALITIES:
+            raise ValueError(f"pmgt_b200 supports 1 to {MAX_MODALITIES} feature modalities; feat_hidden_sizes has "
+                             f"{len(self.feat_hidden_sizes)} entries")
 
     @property
     def use_return_dict(self):

@@ -307,11 +307,10 @@ class GradArena:
 def encoder_param_order(bert: "PMGTModel", prefix: str = "") -> List[Tuple[str, nn.Parameter]]:
     """Flat order of the encoder's trainable parameters (names carry ``prefix``)."""
     e = bert.embeddings
-    out = [
-        ("embeddings.feat_linear.0.weight", e.feat_linear[0].weight),
-        ("embeddings.feat_linear.1.weight", e.feat_linear[1].weight),
-        ("embeddings.feat_linear.0.bias", e.feat_linear[0].bias),
-        ("embeddings.feat_linear.1.bias", e.feat_linear[1].bias),
+    # every feature projection's weight, then every bias (the flat buffer layout of the two-modality model)
+    out = [(f"embeddings.feat_linear.{m}.weight", l.weight) for m, l in enumerate(e.feat_linear)]
+    out += [(f"embeddings.feat_linear.{m}.bias", l.bias) for m, l in enumerate(e.feat_linear)]
+    out += [
         ("embeddings.attention.1.weight", e.attention[1].weight),
         ("embeddings.attention.1.bias", e.attention[1].bias),
         ("embeddings.position_embeddings.weight", e.position_embeddings.weight),
@@ -443,7 +442,7 @@ class _EncoderPlan:
 
 class _EncoderRun:
     """Activations of one encoder pass kept for the backward pass."""
-    __slots__ = ("R", "L", "T", "mask", "rows_idx", "src", "src_rows", "ev", "et", "x0", "layers", "seed", "p_hid",
+    __slots__ = ("R", "L", "T", "mask", "rows_idx", "src", "src_rows", "proj", "x0", "layers", "seed", "p_hid",
                  "p_att", "hidden_f32", "tile", "dense_tables", "last_rows")
 
 
@@ -501,7 +500,7 @@ def _encode_forward(fp: FlatParams, pre: str, cfg: PMGTConfig, src: List[torch.T
     dense_tables = rows_idx is not None and (PROJECTION_MODE == "table" or
                                              (PROJECTION_MODE == "auto" and 4 * src[0].shape[0] <= T))
     proj = []
-    for m in range(2):
+    for m in range(len(src)):
         if dense_tables:
             out = new(src[m].shape[0], H)
             ops.linear_fwd(src[m], fp.bf16(f"{E}feat_linear.{m}.weight"), fp.f32(f"{E}feat_linear.{m}.bias"), out,
@@ -512,18 +511,18 @@ def _encode_forward(fp: FlatParams, pre: str, cfg: PMGTConfig, src: List[torch.T
                            rows=rows_idx, src_rows=(src[m].shape[0] if rows_idx is not None else 0))
         proj.append(out)
     x = new(T, H)
-    ea = ops.embed_args(R, L, H, proj[0], proj[1], fp.f32(E + "attention.1.weight"), fp.f32(E + "attention.1.bias"),
-                        fp.f32(E + "position_embeddings.weight"), fp.f32(E + "role_embeddings.weight"),
-                        fp.f32(E + "LayerNorm.weight"), fp.f32(E + "LayerNorm.bias"), cfg.layer_norm_eps, p_hid, seed, 0,
-                        x_out=x, row_idx=(rows_idx if dense_tables else None))
-    ops.embed_fuse_fwd(ea)
+    ea = ops.embed_multi_args(R, L, H, proj, fp.f32(E + "attention.1.weight"), fp.f32(E + "attention.1.bias"),
+                              fp.f32(E + "position_embeddings.weight"), fp.f32(E + "role_embeddings.weight"),
+                              fp.f32(E + "LayerNorm.weight"), fp.f32(E + "LayerNorm.bias"), cfg.layer_norm_eps, p_hid, seed,
+                              0, x_out=x, row_idx=(rows_idx if dense_tables else None))
+    ops.embed_multi_fwd(ea)
 
     run = None
     if keep:
         run = _EncoderRun()
         run.R, run.L, run.T, run.mask, run.rows_idx = R, L, T, mask, rows_idx
         run.src, run.src_rows = src, [s.shape[0] for s in src]
-        run.ev, run.et, run.x0, run.layers = proj[0], proj[1], x, []
+        run.proj, run.x0, run.layers = proj, x, []
         run.seed, run.p_hid, run.p_att = seed, p_hid, p_att
         run.dense_tables = dense_tables
 
@@ -744,11 +743,12 @@ def _encode_backward(fp: FlatParams, pre: str, cfg: PMGTConfig, run: _EncoderRun
         ops.host_hook(fp.after_layers_hook, arena)
     # ---- embeddings
     E = pre + "embeddings."
+    n_mod = len(run.src)
     common = dict(dx=dy, dx_b=dy_b, d_w_att=G(E + "attention.1.weight"), d_b_att=G(E + "attention.1.bias"),
                   d_pos=G(E + "position_embeddings.weight"), d_role=G(E + "role_embeddings.weight"),
                   d_ln_g=G(E + "LayerNorm.weight"), d_ln_b=G(E + "LayerNorm.bias"),
-                  d_bias_v=G(E + "feat_linear.0.bias"), d_bias_t=G(E + "feat_linear.1.bias"))
-    eargs = (R, L, H, run.ev, run.et, fp.f32(E + "attention.1.weight"), fp.f32(E + "attention.1.bias"),
+                  d_bias=[G(f"{E}feat_linear.{m}.bias") for m in range(n_mod)])
+    eargs = (R, L, H, run.proj, fp.f32(E + "attention.1.weight"), fp.f32(E + "attention.1.bias"),
              fp.f32(E + "position_embeddings.weight"), fp.f32(E + "role_embeddings.weight"),
              fp.f32(E + "LayerNorm.weight"), fp.f32(E + "LayerNorm.bias"), cfg.layer_norm_eps, p_hid, seed, 0)
     if run.dense_tables:
@@ -757,16 +757,15 @@ def _encode_backward(fp: FlatParams, pre: str, cfg: PMGTConfig, run: _EncoderRun
         for acc in accs:
             ops.zero_(acc)
         skip0 = int(all(getattr(t, "_pmgt_row0_zero", False) for t in run.src))
-        ops.embed_fuse_bwd(ops.embed_args(*eargs, row_idx=run.rows_idx, dev_acc=accs[0], det_acc=accs[1], skip_row0=skip0,
-                                          **common))
-        for m in range(2):
+        ops.embed_multi_bwd(ops.embed_multi_args(*eargs, row_idx=run.rows_idx, de_acc=accs, skip_row0=skip0, **common))
+        for m in range(n_mod):
             d16 = new(run.src_rows[m], H)
             ops.cast_f32_bf16(accs[m].view(-1), d16.view(-1))
             ops.linear_dw(d16, run.src[m], G(f"{E}feat_linear.{m}.weight"), tag="gemm_dw_table")
     else:
-        dev_, det_ = new(T, H), new(T, H)
-        ops.embed_fuse_bwd(ops.embed_args(*eargs, dev=dev_, det=det_, **common))
-        for m, d in enumerate((dev_, det_)):
+        des = [new(T, H) for _ in range(n_mod)]
+        ops.embed_multi_bwd(ops.embed_multi_args(*eargs, de=des, **common))
+        for m, d in enumerate(des):
             ops.linear_dw(d, run.src[m], G(f"{E}feat_linear.{m}.weight"), rows=run.rows_idx,
                           src_rows=(run.src_rows[m] if run.rows_idx is not None else 0), x_cols=run.src[m].shape[1])
 
@@ -776,14 +775,14 @@ class _EncodeFn(torch.autograd.Function):
     that autograd routes their gradients; the data is read from ``fp``."""
 
     @staticmethod
-    def forward(ctx, host, src_v, src_t, rows_idx, mask, R, L, training, seed, arena, keep, last_rows, *params):
+    def forward(ctx, host, src, rows_idx, mask, R, L, training, seed, arena, keep, last_rows, *params):
         fp, pre, cfg = host._fp, host._fp_prefix, host.config
-        plan = host._plan_for(fp, [src_v, src_t], rows_idx, R, L, training, keep, arena, last_rows)
+        plan = host._plan_for(fp, src, rows_idx, R, L, training, keep, arena, last_rows)
         host._active_plan = plan
         if plan is not None:
-            hidden, run = plan.forward(fp, pre, cfg, [src_v, src_t], rows_idx, mask, training, seed, keep, last_rows), None
+            hidden, run = plan.forward(fp, pre, cfg, src, rows_idx, mask, training, seed, keep, last_rows), None
         else:
-            hidden, run = _encode_forward(fp, pre, cfg, [src_v, src_t], rows_idx, R, L, mask, training, seed, keep,
+            hidden, run = _encode_forward(fp, pre, cfg, src, rows_idx, R, L, mask, training, seed, keep,
                                           last_rows=last_rows)
         ctx.host, ctx.run, ctx.arena, ctx.n_params, ctx.plan, ctx.keep = host, run, arena, len(params), plan, keep
         return hidden
@@ -802,7 +801,7 @@ class _EncodeFn(torch.autograd.Function):
             _encode_backward(fp, pre, cfg, run, d_hidden, arena)
             ctx.run = None
         grads = tuple(arena.view(n) for n in host._encoder_param_names)
-        return (None,) * 12 + grads
+        return (None,) * 11 + grads
 
 
 class PMGTPretrainedModel(nn.Module):
@@ -905,10 +904,11 @@ class PMGTModel(PMGTPretrainedModel):
             self.__dict__["_encoder_params_cache"] = ps
         return ps
 
-    def encode(self, src_v, src_t, rows_idx, mask, R, L, arena=None, refresh=True, last_rows=None):
-        """``last_rows`` (sorted unique token indices): return only those rows of the final hidden state, as a
-        ``[len(last_rows), H]`` matrix; on the token-tile path the last layer's post-attention half is then computed for
-        those rows only (see ``_encode_forward``)."""
+    def encode(self, src, rows_idx, mask, R, L, arena=None, refresh=True, last_rows=None):
+        """``src``: one bf16 source per modality (feature tables gathered through ``rows_idx``, or dense ``[R * L, D]``
+        matrices when ``rows_idx`` is None).  ``last_rows`` (sorted unique token indices): return only those rows of
+        the final hidden state, as a ``[len(last_rows), H]`` matrix; on the token-tile path the last layer's
+        post-attention half is then computed for those rows only (see ``_encode_forward``)."""
         fp = self._flat()
         if refresh:
             fp.refresh_bf16()
@@ -921,7 +921,10 @@ class PMGTModel(PMGTPretrainedModel):
         cfg = self.config
         in_kernel = (last_rows is not None and cfg.num_hidden_layers > 0
                      and _tile_path(cfg.hidden_size, cfg.intermediate_size))
-        out = _EncodeFn.apply(self, src_v, src_t, rows_idx, mask, R, L, self.training, seed, arena, keep,
+        src = tuple(src)
+        if len(src) != len(cfg.feat_hidden_sizes):
+            raise PMGTError(f"encode: {len(src)} feature sources for {len(cfg.feat_hidden_sizes)} modalities")
+        out = _EncodeFn.apply(self, src, rows_idx, mask, R, L, self.training, seed, arena, keep,
                               last_rows if in_kernel else None, *params)
         if last_rows is not None and not in_kernel:  # other widths: encode everything, then pick the rows
             self._active_plan = None  # the gradient of the picked rows does not line up with the plan's buffer
@@ -930,6 +933,8 @@ class PMGTModel(PMGTPretrainedModel):
 
     def forward(self, *input_feat_embeds, attention_mask=None, head_mask=None, output_attentions=None,
                 output_hidden_states=None, return_dict=None):
+        assert len(input_feat_embeds) == len(self.config.feat_hidden_sizes), \
+            f"# of multi-modal features must be {len(self.config.feat_hidden_sizes)}"
         first = input_feat_embeds[0]
         assert all(first.size()[:-1] == f.size()[:-1] for f in input_feat_embeds[1:]), \
             "All features are same dim except last one"
@@ -943,7 +948,7 @@ class PMGTModel(PMGTPretrainedModel):
         if attention_mask is None:
             attention_mask = torch.ones(R, L, device=first.device)
         dense = [f.reshape(R * L, f.shape[-1]).to(BF16).contiguous() for f in input_feat_embeds]
-        seq = self.encode(dense[0], dense[1], None, attention_mask, R, L)
+        seq = self.encode(dense, None, attention_mask, R, L)
         if not return_dict:
             return (seq, None)
         return BaseModelOutputWithPooling(last_hidden_state=seq, pooler_output=None)

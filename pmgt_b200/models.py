@@ -251,7 +251,7 @@ class PMGT(PMGTPretrainedModel):
             if len(cache) > 8:
                 cache.clear()
             sel = cache[key] = (torch.arange(B, device=ids.device) * L).contiguous()
-        return self.bert.encode(tables[0], tables[1], ids.reshape(-1).contiguous(), mask, B, L, refresh=False, last_rows=sel)
+        return self.bert.encode(tables, ids.reshape(-1).contiguous(), mask, B, L, refresh=False, last_rows=sel)
 
     def prepare_inputs(self, target_node_inputs, pair_node_inputs, num_pairs, masked_inputs) -> Dict[str, torch.Tensor]:
         """Everything ``forward`` derives from the batch alone (training with pairs): the concatenated
@@ -333,7 +333,7 @@ class PMGT(PMGTPretrainedModel):
         ids_flat = ids_flat.contiguous()
         R = mask_all.shape[0]
         if pair_node_inputs is None:
-            hidden = self.bert.encode(tables[0], tables[1], ids_flat, mask_all, R, L,
+            hidden = self.bert.encode(tables, ids_flat, mask_all, R, L,
                                       arena=arena, refresh=False)  # (R, L, H) fp32
             H = hidden.shape[-1]
             last_hidden_state = hidden[:B]
@@ -343,7 +343,7 @@ class PMGT(PMGTPretrainedModel):
             # masked ones).  The encoder prunes its last layer to them and returns the compact [Tc, H] matrix.
             dev = t_ids.device
             sel = self._last_rows(B, SP, L, nfr_on, dev)
-            hidden = self.bert.encode(tables[0], tables[1], ids_flat, mask_all, R, L,
+            hidden = self.bert.encode(tables, ids_flat, mask_all, R, L,
                                       arena=arena, refresh=False, last_rows=sel)  # (Tc, H) fp32
             H = hidden.shape[-1]
             last_hidden_state = hidden[:B * L].view(B, L, H)

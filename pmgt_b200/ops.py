@@ -9,7 +9,7 @@ import ctypes as C
 import torch
 
 from . import _lib
-from ._lib import (AttnArgs, DwTileArgs, EmbedArgs, BlockArgs, GemmArgs, GsrArgs, LinearTileArgs, LnBwdArgs, NfrArgs, ResLnArgs, check,
+from ._lib import (AttnArgs, DwTileArgs, EmbedArgs, EmbedMultiArgs, BlockArgs, GemmArgs, GsrArgs, LinearTileArgs, LnBwdArgs, NfrArgs, ResLnArgs, check,
                    cur_stream, ptr)
 
 EPI_BIAS, EPI_GELU, EPI_GELU_BWD, EPI_ADDEND, EPI_OUT_F32, EPI_ATOMIC = 1, 2, 4, 8, 16, 32
@@ -378,6 +378,41 @@ def embed_fuse_fwd(a: EmbedArgs):
 def embed_fuse_bwd(a: EmbedArgs):
     T = a.rows * a.L
     _run("embed_fuse_bwd", _lib.lib().pmgt_embed_fuse_bwd, (C.byref(a), cur_stream()), 1, 10 * T * a.H)
+
+
+_PER_MODALITY = ("de", "d_bias", "de_acc")
+
+
+def embed_multi_args(rows, L, H, e, w_att, b_att, pos, role, ln_g, ln_b, eps, p, seed, site, **kw):
+    """``pmgt_embed_multi_args`` for ``len(e)`` modalities; ``de`` / ``d_bias`` / ``de_acc`` take one tensor per
+    modality, the other keywords are the fields of ``pmgt_embed_args``."""
+    a = EmbedMultiArgs()
+    if not 1 <= len(e) <= _lib.MAX_MODALITIES:
+        raise _lib.PMGTError(f"embed_multi_args: {len(e)} modalities, supported 1..{_lib.MAX_MODALITIES}")
+    a.rows, a.L, a.H, a.n_mod = rows, L, H, len(e)
+    for m, t in enumerate(e):
+        a.e[m] = ptr(t)
+    a.w_att, a.b_att, a.pos, a.role, a.ln_g, a.ln_b = ptr(w_att), ptr(b_att), ptr(pos), ptr(role), ptr(ln_g), ptr(ln_b)
+    a.ln_eps, a.dropout_p, a.dropout_seed, a.dropout_site = eps, p, seed, site
+    for k, v in kw.items():
+        if k in _PER_MODALITY:
+            arr = getattr(a, k)
+            for m, t in enumerate(v):
+                arr[m] = ptr(t)
+        else:
+            setattr(a, k, v if isinstance(v, (int, bool)) else ptr(v))
+    return a
+
+
+def embed_multi_fwd(a: EmbedMultiArgs):
+    """Embedding fusion for 1..4 modalities (profile tag shared with the two-modality kernel)."""
+    T = a.rows * a.L
+    _run("embed_fuse_fwd", _lib.lib().pmgt_embed_multi_fwd, (C.byref(a), cur_stream()), 1, 2 * (a.n_mod + 1) * T * a.H)
+
+
+def embed_multi_bwd(a: EmbedMultiArgs):
+    T = a.rows * a.L
+    _run("embed_fuse_bwd", _lib.lib().pmgt_embed_multi_bwd, (C.byref(a), cur_stream()), 1, 2 * (2 * a.n_mod + 1) * T * a.H)
 
 
 def attn_args(rows, L, H, heads, beta, qkvc, mask, p, seed, site, **kw):

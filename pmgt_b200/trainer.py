@@ -166,7 +166,7 @@ def init_model(args: AttrDict) -> None:
     if args.graph is None:
         args.graph, args.feat_init_emb = _load_graph_and_features(args)
     feats = args.feat_init_emb
-    config = PMGTConfig(hidden_size=args.hidden_size, feat_hidden_sizes=[int(feats[0].shape[-1]), int(feats[1].shape[-1])],
+    config = PMGTConfig(hidden_size=args.hidden_size, feat_hidden_sizes=[int(f.shape[-1]) for f in feats],
                         intermediate_size=args.intermediate_size, num_hidden_layers=args.num_hidden_layers,
                         num_attention_heads=args.num_attention_heads, beta=args.beta,
                         **({"hidden_dropout_prob": args.hidden_dropout_prob} if args.hidden_dropout_prob is not None else {}),
