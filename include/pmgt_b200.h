@@ -295,7 +295,7 @@ int pmgt_gather_proj_dw(const pmgt_gather_proj_args* a, void* stream);
 /* ------------------------------------------------------------------------ */
 /*
  * Dual-softmax "diversity promoting" attention core of PMGTSelfAttention
- * (modeling_pmgt.py:435-526), one (sequence, head) per warp:
+ * (modeling_pmgt.py:435-526), per (sequence, head):
  *   S1 = 1 - C C^T / (|C||C|^T) + I + mask ; P1 = dropout(softmax(S1))
  *   S2 = Q K^T / sqrt(dh) + mask           ; P2 = dropout(softmax(S2))
  *   ctx = (beta P1 + (1-beta) P2) V
@@ -304,6 +304,11 @@ int pmgt_gather_proj_dw(const pmgt_gather_proj_args* a, void* stream);
  * of transformers 4.11.2 get_extended_attention_mask is applied inside).
  * Backward recomputes P1/P2 and writes dqkvc [T][4H] bf16 and accumulates the
  * bias gradient d_bias_qkvc [4H] (fp32 atomicAdd) when non-NULL.
+ * qkvc, ctx (forward), dctx and dqkvc (backward) must be 16-byte aligned;
+ * otherwise the call returns PMGT_ERR_INVALID.  1 <= L <= 128, even head size.
+ * The kernel, and with it the dropout stream, depends only on the shape
+ * (L, H, heads, rows * heads), so a forward / backward pair with the same
+ * dropout_seed and dropout_site always sees the same mask.
  */
 typedef struct pmgt_attn_args {
   int64_t rows; int L; int H; int heads; float beta;

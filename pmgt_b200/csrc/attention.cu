@@ -1,11 +1,19 @@
 // K3 attention core: the dual-softmax "diversity promoting" self-attention of
 // PMGTSelfAttention.forward (pmgt/pmgt/modeling_pmgt.py:435-526), forward and
-// backward, for very short sequences (L = max_ctx_neigh + 1, 6 by default).
+// backward, over sequences of L = max_ctx_neigh + 1 tokens (6 by default).
 //
-// One warp owns one (sequence, head).  Q/K/V/C rows of that head are staged in
-// a per-warp shared-memory tile (bf16, row stride dh+2 to stay bank-conflict
-// free), the L x L score matrices live in shared memory as fp32, and the
-// (i, j) pairs / the dh columns are spread over the 32 lanes.
+// pmgt_attn_core_fwd / _bwd validate the arguments and pick one kernel family
+// from the shape alone (attn_family):
+//   attn_mma  (attention_mma.cu)  L = 6,           head size 32 / 64 / 128
+//   attn_reg  (attention_reg.cu)  8 < L <= 64,     head size 32 / 64 / 128
+//   attn_mid  (attention_mid.cu)  8 < L <= 64,     other head sizes that are a multiple of 16, if its
+//                                                  backward shared-memory layout fits
+//   generic   (this file)         everything else, L <= 128, even head size
+//
+// The generic kernel: one warp owns one (sequence, head).  Q/K/V/C rows of that
+// head are staged in a per-warp shared-memory tile (bf16, row stride dh+2 to stay
+// bank-conflict free), the L x L score matrices live in shared memory as fp32,
+// and the (i, j) pairs / the dh columns are spread over the 32 lanes.
 //
 //   G   = C C^T,  n_i = sqrt(G_ii)
 //   S1  = 1 - G / (n n^T) + I + maskadd     P1 = dropout(softmax(S1))
@@ -285,31 +293,74 @@ __global__ void __launch_bounds__(128) attn_core_bwd_kernel(const pmgt_attn_args
   }
 }
 
-static int attn_launch_cfg(const pmgt_attn_args* a, bool bwd, AttnSmemLayout& lay, int& warps, size_t& smem) {
-  PMGT_REQUIRE(a->heads >= 1 && a->H % a->heads == 0, "attention: H must be divisible by heads");
+static int attn_generic(const pmgt_attn_args* a, bool bwd, cudaStream_t st) {
   const int dh = a->H / a->heads;
-  PMGT_REQUIRE(dh % 2 == 0, "attention: head size must be even");
-  PMGT_REQUIRE(a->L >= 1 && a->L <= 128, "attention: L must be in [1,128]");
-  lay = attn_layout(a->L, dh);
+  const AttnSmemLayout lay = attn_layout(a->L, dh);
   const size_t per = bwd ? lay.per_warp_bwd : lay.per_warp_fwd;
   const size_t budget = 200 * 1024;
   PMGT_REQUIRE(per <= budget, "attention: L=%d, head size %d needs %zu bytes of shared memory per warp (> %zu)", a->L, dh,
                per, budget);
-  warps = (int)(budget / per);
+  int warps = (int)(budget / per);
   if (warps > 4) warps = 4;
-  // keep at least ~4 CTAs resident per SM when tiles are small
-  smem = per * warps;
+  const size_t smem = per * warps;
+  if (smem > 48 * 1024) {
+    if (bwd) PMGT_CHECK_CUDA(cudaFuncSetAttribute(attn_core_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    else PMGT_CHECK_CUDA(cudaFuncSetAttribute(attn_core_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  }
+  const long long items = a->rows * a->heads;
+  long long ctas = (items + warps - 1) / warps;
+  const long long cap = (long long)num_sms() * 8;
+  if (ctas > cap) ctas = cap;
+  if (bwd) attn_core_bwd_kernel<<<(unsigned)ctas, 128, smem, st>>>(*a, warps, lay);
+  else attn_core_fwd_kernel<<<(unsigned)ctas, 128, smem, st>>>(*a, warps, lay);
+  PMGT_LAUNCH_CHECK();
   return PMGT_OK;
 }
 
-int attn_small_fwd(const pmgt_attn_args* a, cudaStream_t st);  // attention_small.cu
-int attn_small_bwd(const pmgt_attn_args* a, cudaStream_t st);
-int attn_mma_fwd(const pmgt_attn_args* a, cudaStream_t st);    // attention_mma.cu
+// Launchers of the other kernel families; each assumes attn_family() chose it.
+int attn_mma_fwd(const pmgt_attn_args* a, cudaStream_t st);  // attention_mma.cu
 int attn_mma_bwd(const pmgt_attn_args* a, cudaStream_t st);
-int attn_reg_fwd(const pmgt_attn_args* a, cudaStream_t st);    // attention_reg.cu (8 < L <= 64, scores in MMA fragments)
+int attn_reg_fwd(const pmgt_attn_args* a, cudaStream_t st);  // attention_reg.cu
 int attn_reg_bwd(const pmgt_attn_args* a, cudaStream_t st);
-int attn_mid_fwd(const pmgt_attn_args* a, cudaStream_t st);    // attention_mid.cu (8 < L <= 64, tensor-core products)
+int attn_mid_fwd(const pmgt_attn_args* a, cudaStream_t st);  // attention_mid.cu
 int attn_mid_bwd(const pmgt_attn_args* a, cudaStream_t st);
+bool attn_mid_fits(int L, int dh);
+
+enum class AttnFamily { Mma, Reg, Mid, Generic };
+
+// The table at the top of this file.  Only the shape decides, not pointers and not the direction, so the backward pass
+// runs the family of its forward pass and regenerates the dropout mask that one drew (attn_reg has a stream of its
+// own).  The head sizes below are multiples of 16, so H is a multiple of 8 and, with the base pointers 16-byte aligned
+// (attn_check), so is every row the tensor-core families stage.
+static AttnFamily attn_family(const pmgt_attn_args* a) {
+  const int L = a->L, dh = a->H / a->heads;
+  const bool reg_dh = dh == 32 || dh == 64 || dh == 128;
+  if (L == 6 && reg_dh) return AttnFamily::Mma;
+  if (L > 8 && L <= 64) {
+    if (reg_dh && a->rows * a->heads <= 0x7fffffffll) return AttnFamily::Reg;  // one CTA per (sequence, head)
+    if (dh % 16 == 0 && attn_mid_fits(L, dh)) return AttnFamily::Mid;
+  }
+  return AttnFamily::Generic;
+}
+
+static bool misaligned16(const void* p) { return ((uintptr_t)p & 15) != 0; }
+
+// the argument checks of both entry points, made before any CUDA call
+static int attn_check(const pmgt_attn_args* a, bool bwd) {
+  const char* fn = bwd ? "pmgt_attn_core_bwd" : "pmgt_attn_core_fwd";
+  PMGT_REQUIRE(a && a->qkvc && a->mask && (bwd ? a->dctx && a->dqkvc : a->ctx != nullptr), "%s: null argument", fn);
+  PMGT_REQUIRE(!misaligned16(a->qkvc), "%s: qkvc must be 16-byte aligned", fn);
+  if (bwd) {
+    PMGT_REQUIRE(!misaligned16(a->dctx), "%s: dctx must be 16-byte aligned", fn);
+    PMGT_REQUIRE(!misaligned16(a->dqkvc), "%s: dqkvc must be 16-byte aligned", fn);
+  } else {
+    PMGT_REQUIRE(!misaligned16(a->ctx), "%s: ctx must be 16-byte aligned", fn);
+  }
+  PMGT_REQUIRE(a->heads >= 1 && a->H % a->heads == 0, "attention: H must be divisible by heads");
+  PMGT_REQUIRE((a->H / a->heads) % 2 == 0, "attention: head size must be even");
+  PMGT_REQUIRE(a->L >= 1 && a->L <= 128, "attention: L must be in [1,128]");
+  return PMGT_OK;
+}
 
 }  // namespace pmgt
 
@@ -318,58 +369,29 @@ using namespace pmgt;
 extern "C" {
 
 int pmgt_attn_core_fwd(const pmgt_attn_args* a, void* stream) {
-  PMGT_REQUIRE(a && a->qkvc && a->mask && a->ctx, "pmgt_attn_core_fwd: null argument");
-  if (a->rows == 0) return PMGT_OK;
-  PMGT_REQUIRE(a->heads >= 1 && a->H % a->heads == 0, "attention: H must be divisible by heads");
-  {  // register-resident kernel for the short-sequence shapes (default PMGT: L = 6, dh = 128)
-    int r = attn_mma_fwd(a, (cudaStream_t)stream);
-    if (r == 0) r = attn_small_fwd(a, (cudaStream_t)stream);
-    if (r == 0) r = attn_reg_fwd(a, (cudaStream_t)stream);
-    if (r == 0) r = attn_mid_fwd(a, (cudaStream_t)stream);
-    if (r < 0) return r;
-    if (r > 0) return PMGT_OK;
+  const int rc = attn_check(a, false);
+  if (rc || a->rows == 0) return rc;
+  const cudaStream_t st = (cudaStream_t)stream;
+  switch (attn_family(a)) {
+    case AttnFamily::Mma: return attn_mma_fwd(a, st);
+    case AttnFamily::Reg: return attn_reg_fwd(a, st);
+    case AttnFamily::Mid: return attn_mid_fwd(a, st);
+    default: return attn_generic(a, false, st);
   }
-  AttnSmemLayout lay; int warps; size_t smem;
-  int rc = attn_launch_cfg(a, false, lay, warps, smem);
-  if (rc) return rc;
-  if (smem > 48 * 1024)
-    PMGT_CHECK_CUDA(cudaFuncSetAttribute(attn_core_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  long long items = a->rows * a->heads;
-  long long ctas = (items + warps - 1) / warps;
-  long long cap = (long long)num_sms() * 8;
-  if (ctas > cap) ctas = cap;
-  attn_core_fwd_kernel<<<(unsigned)ctas, 128, smem, (cudaStream_t)stream>>>(*a, warps, lay);
-  PMGT_LAUNCH_CHECK();
-  return PMGT_OK;
 }
 
 int pmgt_attn_core_bwd(const pmgt_attn_args* a, void* stream) {
-  PMGT_REQUIRE(a && a->qkvc && a->mask && a->dctx && a->dqkvc, "pmgt_attn_core_bwd: null argument");
-  if (a->rows == 0) return PMGT_OK;
-  PMGT_REQUIRE(a->heads >= 1 && a->H % a->heads == 0, "attention: H must be divisible by heads");
-  int rc = attn_mma_bwd(a, (cudaStream_t)stream);
-  if (rc == 0) rc = attn_small_bwd(a, (cudaStream_t)stream);
-  if (rc == 0) rc = attn_reg_bwd(a, (cudaStream_t)stream);
-  if (rc == 0) rc = attn_mid_bwd(a, (cudaStream_t)stream);
-  if (rc < 0) return rc;
-  if (rc == 0) {
-    AttnSmemLayout lay; int warps; size_t smem;
-    rc = attn_launch_cfg(a, true, lay, warps, smem);
-    if (rc) return rc;
-    if (smem > 48 * 1024)
-      PMGT_CHECK_CUDA(cudaFuncSetAttribute(attn_core_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    long long items = a->rows * a->heads;
-    long long ctas = (items + warps - 1) / warps;
-    long long cap = (long long)num_sms() * 8;
-    if (ctas > cap) ctas = cap;
-    attn_core_bwd_kernel<<<(unsigned)ctas, 128, smem, (cudaStream_t)stream>>>(*a, warps, lay);
-    PMGT_LAUNCH_CHECK();
+  int rc = attn_check(a, true);
+  if (rc || a->rows == 0) return rc;
+  const cudaStream_t st = (cudaStream_t)stream;
+  switch (attn_family(a)) {
+    case AttnFamily::Mma: rc = attn_mma_bwd(a, st); break;
+    case AttnFamily::Reg: rc = attn_reg_bwd(a, st); break;
+    case AttnFamily::Mid: rc = attn_mid_bwd(a, st); break;
+    default: rc = attn_generic(a, true, st);
   }
-  if (a->d_bias_qkvc) {
-    rc = pmgt_colsum_bf16(a->dqkvc, a->rows * a->L, 4ll * a->H, 4ll * a->H, a->d_bias_qkvc, stream);
-    if (rc) return rc;
-  }
-  return PMGT_OK;
+  if (rc == PMGT_OK && a->d_bias_qkvc) rc = pmgt_colsum_bf16(a->dqkvc, a->rows * a->L, 4ll * a->H, 4ll * a->H, a->d_bias_qkvc, stream);
+  return rc;
 }
 
 }  // extern "C"

@@ -364,48 +364,35 @@ __global__ void __launch_bounds__(kMidThreads) attn_mid_bwd_kernel(const pmgt_at
   }
 }
 
-// shared memory of one CTA (= one item in flight) and how many CTAs fit per SM
-int mid_cfg(const pmgt_attn_args* a, bool bwd, MidLayout& lay, size_t& smem, int& per_sm) {
-  lay = mid_layout(a->L, a->H / a->heads);
-  smem = bwd ? lay.per_warp_bwd : lay.per_warp_fwd;
-  if (smem > 220 * 1024) return 0;
-  per_sm = (int)((224 * 1024) / (smem + 1024));
+constexpr size_t kMidSmemMax = 220 * 1024;  // shared memory of one CTA (= one item in flight)
+
+template <bool BWD>
+int launch_mid(const pmgt_attn_args* a, cudaStream_t st) {
+  const MidLayout lay = mid_layout(a->L, a->H / a->heads);
+  const size_t smem = BWD ? lay.per_warp_bwd : lay.per_warp_fwd;
+  static unsigned long long configured = 0;
+  if (first_use_on_device(configured)) {
+    if (BWD) PMGT_CHECK_CUDA(cudaFuncSetAttribute(attn_mid_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMidSmemMax));
+    else PMGT_CHECK_CUDA(cudaFuncSetAttribute(attn_mid_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMidSmemMax));
+  }
+  int per_sm = (int)((224 * 1024) / (smem + 1024));  // CTAs that fit per SM
   if (per_sm > 16) per_sm = 16;
   if (per_sm < 1) per_sm = 1;
-  return 1;
+  const long long items = a->rows * a->heads;
+  long long ctas = (long long)num_sms() * per_sm;
+  if (ctas > items) ctas = items;
+  if (BWD) attn_mid_bwd_kernel<<<(unsigned)ctas, kMidThreads, smem, st>>>(*a, lay);
+  else attn_mid_fwd_kernel<<<(unsigned)ctas, kMidThreads, smem, st>>>(*a, lay);
+  PMGT_LAUNCH_CHECK();
+  return PMGT_OK;
 }
 
 }  // namespace
 
-// returns 1 if the shape was handled here, 0 if the caller must use another kernel, < 0 on error
-int attn_mid_fwd(const pmgt_attn_args* a, cudaStream_t st) {
-  const int dh = a->H / a->heads;
-  if (a->L <= 8 || a->L > 64 || dh % 16 != 0 || a->H % 8 != 0) return 0;
-  if ((((uintptr_t)a->qkvc | (uintptr_t)a->ctx) & 15) != 0) return 0;
-  MidLayout lay; size_t smem; int per_sm;
-  if (!mid_cfg(a, false, lay, smem, per_sm)) return 0;
-  PMGT_CHECK_CUDA(cudaFuncSetAttribute(attn_mid_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const long long items = a->rows * a->heads;
-  long long ctas = (long long)num_sms() * per_sm;
-  if (ctas > items) ctas = items;
-  attn_mid_fwd_kernel<<<(unsigned)ctas, kMidThreads, smem, st>>>(*a, lay);
-  PMGT_LAUNCH_CHECK();
-  return 1;
-}
+// Whether the mid kernels take (L, dh): the backward layout, the larger one, decides for both directions.
+bool attn_mid_fits(int L, int dh) { return mid_layout(L, dh).per_warp_bwd <= kMidSmemMax; }
 
-int attn_mid_bwd(const pmgt_attn_args* a, cudaStream_t st) {
-  const int dh = a->H / a->heads;
-  if (a->L <= 8 || a->L > 64 || dh % 16 != 0 || a->H % 8 != 0) return 0;
-  if ((((uintptr_t)a->qkvc | (uintptr_t)a->dctx | (uintptr_t)a->dqkvc) & 15) != 0) return 0;
-  MidLayout lay; size_t smem; int per_sm;
-  if (!mid_cfg(a, true, lay, smem, per_sm)) return 0;
-  PMGT_CHECK_CUDA(cudaFuncSetAttribute(attn_mid_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const long long items = a->rows * a->heads;
-  long long ctas = (long long)num_sms() * per_sm;
-  if (ctas > items) ctas = items;
-  attn_mid_bwd_kernel<<<(unsigned)ctas, kMidThreads, smem, st>>>(*a, lay);
-  PMGT_LAUNCH_CHECK();
-  return 1;
-}
+int attn_mid_fwd(const pmgt_attn_args* a, cudaStream_t st) { return launch_mid<false>(a, st); }
+int attn_mid_bwd(const pmgt_attn_args* a, cudaStream_t st) { return launch_mid<true>(a, st); }
 
 }  // namespace pmgt

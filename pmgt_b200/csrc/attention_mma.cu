@@ -3,7 +3,8 @@
 // The dual-softmax attention of PMGTSelfAttention (pmgt/pmgt/modeling_pmgt.py:435-526; formulas in
 // attention.cu) on a 6-token sequence is a handful of [6 x dh] x [dh x 6] and [6 x 6] x [6 x dh] products per
 // (sequence, head): far below the 64/128-row tiles of tcgen05, and as scalar FMAs they were instruction-bound
-// (attention_small.cu: 27 % of the HBM roofline in backward).  Here one warp owns one (sequence, head):
+// (the scalar kernel this one replaced reached 27 % of the HBM roofline in backward).  Here one warp owns one
+// (sequence, head):
 //   * the Q/K/V/C (and dctx) rows are staged with 16-byte cp.async into a padded shared-memory tile,
 //     double-buffered so the next item streams in while the current one is computed;
 //   * every product runs as m16n8k16 bf16 MMAs with fp32 accumulation (ldmatrix / ldmatrix.trans operand
@@ -12,8 +13,6 @@
 //     fragment layout: lane (g, t) holds row g, columns 2t and 2t+1, so row reductions are two quad shuffles
 //     and an accumulator fragment IS the A operand of the next product (movmatrix for the transposed ones).
 // The kernel is then bound by HBM: forward 10*H, backward 18*H bytes per token.
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace pmgt {
@@ -470,29 +469,15 @@ static int launch_mma(const pmgt_attn_args* a, cudaStream_t st) {
   return PMGT_OK;
 }
 
-// returns 1 if the shape was handled here, 0 if the caller must use another kernel, < 0 on error
+// L = 6, head size 32 / 64 / 128 (attn_family in attention.cu)
 template <bool BWD>
 static int dispatch_mma(const pmgt_attn_args* a, cudaStream_t st) {
-  static int enabled = -1;
-  if (enabled < 0) {
-    const char* e = getenv("PMGT_ATTN_MMA");
-    enabled = (e && e[0] == '0') ? 0 : 1;
-  }
-  if (!enabled) return 0;
   const int dh = a->H / a->heads;
-  if ((a->H % 8) != 0) return 0;
-  if ((((uintptr_t)a->qkvc | (uintptr_t)(BWD ? (const void*)a->dctx : (const void*)a->ctx)) & 15) != 0) return 0;
-  if (BWD && (((uintptr_t)a->dqkvc) & 15) != 0) return 0;
-#define PMGT_ATTN_CASE(L_, DH_)                          \
-  if (a->L == L_ && dh == DH_) {                         \
-    const int r = launch_mma<L_, DH_, BWD>(a, st);       \
-    return r ? r : 1;                                    \
-  }
-  PMGT_ATTN_CASE(6, 128)
-  PMGT_ATTN_CASE(6, 64)
-  PMGT_ATTN_CASE(6, 32)
-#undef PMGT_ATTN_CASE
-  return 0;
+  if (a->L == 6 && dh == 128) return launch_mma<6, 128, BWD>(a, st);
+  if (a->L == 6 && dh == 64) return launch_mma<6, 64, BWD>(a, st);
+  if (a->L == 6 && dh == 32) return launch_mma<6, 32, BWD>(a, st);
+  set_error("attn_mma: no kernel for L=%d, head size %d", a->L, dh);
+  return PMGT_ERR_INVALID;
 }
 
 int attn_mma_fwd(const pmgt_attn_args* a, cudaStream_t st) { return dispatch_mma<false>(a, st); }

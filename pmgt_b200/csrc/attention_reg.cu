@@ -500,33 +500,29 @@ int launch_reg(const pmgt_attn_args* a, cudaStream_t st) {
     if (BWD) PMGT_CHECK_CUDA(cudaFuncSetAttribute(attn_reg_bwd_kernel<DH, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     else PMGT_CHECK_CUDA(cudaFuncSetAttribute(attn_reg_fwd_kernel<DH, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   }
-  const long long items = a->rows * a->heads;
-  if (items > 0x7fffffffll) return 0;
+  const long long items = a->rows * a->heads;  // <= 2^31 - 1 (attn_family in attention.cu)
   if (BWD) attn_reg_bwd_kernel<DH, MT><<<(unsigned)items, 32 * MT, smem, st>>>(*a);
   else attn_reg_fwd_kernel<DH, MT><<<(unsigned)items, 32 * MT, smem, st>>>(*a);
   PMGT_LAUNCH_CHECK();
-  return 1;
+  return PMGT_OK;
 }
 
+// 8 < L <= 64, head size 32 / 64 / 128
 template <bool BWD>
 int dispatch_reg(const pmgt_attn_args* a, cudaStream_t st) {
   const int dh = a->H / a->heads;
-  if (a->L <= 8 || a->L > 64 || a->H % 8 != 0) return 0;
-  if ((((uintptr_t)a->qkvc) & 15) != 0) return 0;
-  if (BWD && ((((uintptr_t)a->dctx | (uintptr_t)a->dqkvc) & 15) != 0)) return 0;
-  if (!BWD && (((uintptr_t)a->ctx) & 3) != 0) return 0;
-  const int mt = (a->L + 15) / 16;
+  const int mt = a->L > 8 && a->L <= 64 ? (a->L + 15) / 16 : 0;
 #define PMGT_REG_CASE(D, M) if (dh == D && mt == M) return launch_reg<D, M, BWD>(a, st)
   PMGT_REG_CASE(32, 1); PMGT_REG_CASE(32, 2); PMGT_REG_CASE(32, 3); PMGT_REG_CASE(32, 4);
   PMGT_REG_CASE(64, 1); PMGT_REG_CASE(64, 2); PMGT_REG_CASE(64, 3); PMGT_REG_CASE(64, 4);
   PMGT_REG_CASE(128, 1); PMGT_REG_CASE(128, 2); PMGT_REG_CASE(128, 3); PMGT_REG_CASE(128, 4);
 #undef PMGT_REG_CASE
-  return 0;
+  set_error("attn_reg: no kernel for L=%d, head size %d", a->L, dh);
+  return PMGT_ERR_INVALID;
 }
 
 }  // namespace
 
-// returns 1 if the shape was handled here, 0 if the caller must use another kernel, < 0 on error
 int attn_reg_fwd(const pmgt_attn_args* a, cudaStream_t st) { return dispatch_reg<false>(a, st); }
 int attn_reg_bwd(const pmgt_attn_args* a, cudaStream_t st) { return dispatch_reg<true>(a, st); }
 

@@ -67,6 +67,27 @@ def test_argument_validation_without_a_gpu(lib):
     assert lib.pmgt_sample_contexts(None, None, None, 0, None, 3, 5, 0, None, None, None, None) == -1
 
 
+def test_attention_rejects_misaligned_buffers_without_a_gpu(lib):
+    """qkvc / ctx / dctx / dqkvc must be 16-byte aligned: a misaligned one is named in the error, before any CUDA call.
+    The pointers are fake, so this only runs where no device could be reached by a faulty check."""
+    import torch
+    if torch.cuda.is_available():
+        pytest.skip("GPU present")
+    from pmgt_b200 import _lib
+    a = _lib.AttnArgs()
+    a.rows, a.L, a.H, a.heads, a.beta = 4, 33, 64, 1, 0.5
+    a.qkvc, a.mask, a.ctx, a.dctx, a.dqkvc = 16, 16, 24, 16, 16
+    a.dropout_p = 0.1
+    assert lib.pmgt_attn_core_fwd(ctypes.byref(a), None) == -1
+    assert b"pmgt_attn_core_fwd: ctx must be 16-byte aligned" in lib.pmgt_last_error()
+    a.dctx = 24
+    assert lib.pmgt_attn_core_bwd(ctypes.byref(a), None) == -1
+    assert b"pmgt_attn_core_bwd: dctx must be 16-byte aligned" in lib.pmgt_last_error()
+    a.dctx, a.dqkvc = 16, 24
+    assert lib.pmgt_attn_core_bwd(ctypes.byref(a), None) == -1
+    assert b"pmgt_attn_core_bwd: dqkvc must be 16-byte aligned" in lib.pmgt_last_error()
+
+
 def test_no_cpu_fallback():
     """Without a CUDA device the product path raises instead of computing on the CPU."""
     import torch

@@ -206,13 +206,14 @@ def test_attention_core_fwd_bwd(R, L, H, heads, beta):
     _close(dbias, dqkvc.float().sum(0), 1e-3, "d_bias_qkvc")
 
 
-@pytest.mark.parametrize("L,dh", [(33, 64), (20, 32), (64, 128)])
-def test_attention_dropout_mask_agrees_between_fwd_and_bwd_medium_L(L, dh):
-    """Register-resident attention core (attention_reg.cu), train mode: with V = the first L unit vectors the forward
-    output rows ARE the dropped attention matrix A; the backward pass (which regenerates the mask in the transposed
+@pytest.mark.parametrize("L,dh", [(33, 64), (20, 32), (64, 128),  # attn_reg
+                                  (6, 128), (33, 48), (70, 128)])  # attn_mma, attn_mid, generic
+def test_attention_dropout_mask_agrees_between_fwd_and_bwd(L, dh):
+    """Attention core in train mode, one shape per kernel family: with V = the first L unit vectors the forward output
+    rows ARE the dropped attention matrix A; the backward pass (which regenerates the mask, attn_reg in the transposed
     orientation) must see the same A: dV_j[c] = A_{i j} for dctx = e_c at row i.  Also the keep rate."""
     ops = _ops()
-    R, H, heads, p = 6, dh, 1, 0.25
+    R, H, heads, p = max(6, 2048 // (L * L)), dh, 1, 0.25  # >= 2048 dropout draws for the keep-rate check
     T = R * L
     qkvc = _r(T, 4 * H, s=0.7)
     v = torch.zeros(R, L, H, device="cuda")
@@ -236,6 +237,29 @@ def test_attention_dropout_mask_agrees_between_fwd_and_bwd_medium_L(L, dh):
         ops.attn_core_bwd(ops.attn_args(R, L, H, heads, 1.0, qkvc, mask, p, 77, 3, dctx=dctx.view(T, H).to(BF16), dqkvc=dqkvc))
         dV = dqkvc[:, 2 * H:3 * H].float().view(R, L, H)[:, :, 5]     # dV[r, j] = A[r, i*, j]
         assert torch.allclose(dV, A[:, i_star, :], rtol=2e-2, atol=2e-3), (i_star, float((dV - A[:, i_star, :]).abs().max()))
+
+
+@pytest.mark.parametrize("which", ["ctx", "dctx", "dqkvc"])
+def test_attention_rejects_misaligned_buffers(which):
+    """qkvc / ctx / dctx / dqkvc must be 16-byte aligned.  A view 8 bytes into a buffer is rejected and named, whichever
+    kernel the shape selects, instead of switching kernels (which changed the dropout stream between fwd and bwd)."""
+    from pmgt_b200._lib import PMGTError
+    ops = _ops()
+    R, L, H, heads, p = 4, 33, 768, 12, 0.1  # attn_reg
+    T = R * L
+    qkvc = _r(T, 4 * H, s=0.7)
+    mask = torch.ones(R, L, device="cuda")
+    bufs = dict(ctx=torch.empty(T, H, device="cuda", dtype=BF16), dctx=_r(T, H), dqkvc=torch.empty_like(qkvc))
+    t = bufs[which]
+    bufs[which] = torch.empty(t.numel() + 4, device="cuda", dtype=BF16)[4:4 + t.numel()].view(t.shape).copy_(t)
+    assert bufs[which].data_ptr() % 16 == 8
+    with pytest.raises(PMGTError, match=f"{which} must be 16-byte aligned"):
+        if which == "ctx":
+            ops.attn_core_fwd(ops.attn_args(R, L, H, heads, 0.5, qkvc, mask, p, 7, 3, ctx=bufs["ctx"]))
+        else:
+            ops.attn_core_bwd(ops.attn_args(R, L, H, heads, 0.5, qkvc, mask, p, 7, 3, dctx=bufs["dctx"],
+                                            dqkvc=bufs["dqkvc"]))
+    torch.cuda.synchronize()
 
 
 @pytest.mark.parametrize("T,H", [(50, 128), (33, 64), (20, 768), (9, 32), (5001, 768), (3000, 256), (1300, 1024), (77, 512)])
