@@ -8,7 +8,8 @@
 //   attn_reg  (attention_reg.cu)  8 < L <= 64,     head size 32 / 64 / 128
 //   attn_mid  (attention_mid.cu)  8 < L <= 64,     other head sizes that are a multiple of 16, if its
 //                                                  backward shared-memory layout fits
-//   generic   (this file)         everything else, L <= 128, even head size
+//   attn_long (attention_long.cu) 64 < L <= 128,   head size 32 / 64 / 128
+//   generic   (this file)         everything else, L <= 128, even head size (within its shared-memory budget)
 //
 // The generic kernel: one warp owns one (sequence, head).  Q/K/V/C rows of that
 // head are staged in a per-warp shared-memory tile (bf16, row stride dh+2 to stay
@@ -325,8 +326,10 @@ int attn_reg_bwd(const pmgt_attn_args* a, cudaStream_t st);
 int attn_mid_fwd(const pmgt_attn_args* a, cudaStream_t st);  // attention_mid.cu
 int attn_mid_bwd(const pmgt_attn_args* a, cudaStream_t st);
 bool attn_mid_fits(int L, int dh);
+int attn_long_fwd(const pmgt_attn_args* a, cudaStream_t st);  // attention_long.cu
+int attn_long_bwd(const pmgt_attn_args* a, cudaStream_t st);
 
-enum class AttnFamily { Mma, Reg, Mid, Generic };
+enum class AttnFamily { Mma, Reg, Mid, Long, Generic };
 
 // The table at the top of this file.  Only the shape decides, not pointers and not the direction, so the backward pass
 // runs the family of its forward pass and regenerates the dropout mask that one drew (attn_reg has a stream of its
@@ -340,6 +343,7 @@ static AttnFamily attn_family(const pmgt_attn_args* a) {
     if (reg_dh && a->rows * a->heads <= 0x7fffffffll) return AttnFamily::Reg;  // one CTA per (sequence, head)
     if (dh % 16 == 0 && attn_mid_fits(L, dh)) return AttnFamily::Mid;
   }
+  if (L > 64 && L <= 128 && reg_dh && a->rows * a->heads <= 0x7fffffffll) return AttnFamily::Long;  // one CTA per (sequence, head)
   return AttnFamily::Generic;
 }
 
@@ -376,6 +380,7 @@ int pmgt_attn_core_fwd(const pmgt_attn_args* a, void* stream) {
     case AttnFamily::Mma: return attn_mma_fwd(a, st);
     case AttnFamily::Reg: return attn_reg_fwd(a, st);
     case AttnFamily::Mid: return attn_mid_fwd(a, st);
+    case AttnFamily::Long: return attn_long_fwd(a, st);
     default: return attn_generic(a, false, st);
   }
 }
@@ -388,6 +393,7 @@ int pmgt_attn_core_bwd(const pmgt_attn_args* a, void* stream) {
     case AttnFamily::Mma: rc = attn_mma_bwd(a, st); break;
     case AttnFamily::Reg: rc = attn_reg_bwd(a, st); break;
     case AttnFamily::Mid: rc = attn_mid_bwd(a, st); break;
+    case AttnFamily::Long: rc = attn_long_bwd(a, st); break;
     default: rc = attn_generic(a, true, st);
   }
   if (rc == PMGT_OK && a->d_bias_qkvc) rc = pmgt_colsum_bf16(a->dqkvc, a->rows * a->L, 4ll * a->H, 4ll * a->H, a->d_bias_qkvc, stream);

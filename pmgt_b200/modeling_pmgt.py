@@ -304,6 +304,18 @@ class GradArena:
         return torch.as_strided(self.get(), shape, strides, off)
 
 
+MAX_CONTEXT_LEN = 128  # the attention core's longest sequence (pmgt_attn_core_fwd / _bwd)
+
+
+def check_context_len(config, L: int) -> None:
+    """A context of ``L`` tokens needs ``L`` rows of the position table and an attention core that covers ``L``."""
+    if L > config.max_position_embeddings:
+        raise ValueError(f"context of {L} tokens exceeds the position table: max_position_embeddings is "
+                         f"{config.max_position_embeddings}")
+    if L > MAX_CONTEXT_LEN:
+        raise ValueError(f"context of {L} tokens exceeds the attention core's limit of {MAX_CONTEXT_LEN} tokens")
+
+
 def encoder_param_order(bert: "PMGTModel", prefix: str = "") -> List[Tuple[str, nn.Parameter]]:
     """Flat order of the encoder's trainable parameters (names carry ``prefix``)."""
     e = bert.embeddings
@@ -908,7 +920,11 @@ class PMGTModel(PMGTPretrainedModel):
         """``src``: one bf16 source per modality (feature tables gathered through ``rows_idx``, or dense ``[R * L, D]``
         matrices when ``rows_idx`` is None).  ``last_rows`` (sorted unique token indices): return only those rows of
         the final hidden state, as a ``[len(last_rows), H]`` matrix; on the token-tile path the last layer's
-        post-attention half is then computed for those rows only (see ``_encode_forward``)."""
+        post-attention half is then computed for those rows only (see ``_encode_forward``).
+
+        Raises ``ValueError``, before any device work, for a context longer than the position table or than the
+        attention core's limit (MAX_CONTEXT_LEN tokens)."""
+        check_context_len(self.config, L)
         fp = self._flat()
         if refresh:
             fp.refresh_bf16()

@@ -104,6 +104,11 @@ def check_args(args: AttrDict) -> None:
                          "fp32 accumulation")
     if args.accumulation_step is not None and int(args.accumulation_step) < 1:
         raise ValueError("accumulation_step must be >= 1")
+    # init_model builds the config with the default position table: a context is max_ctx_neigh + 1 tokens
+    max_pos = PMGTConfig().max_position_embeddings
+    if int(args.max_ctx_neigh) + 1 > max_pos:
+        raise ValueError(f"max_ctx_neigh must be <= {max_pos - 1}: a context of max_ctx_neigh + 1 tokens needs that "
+                         f"many rows of the {max_pos}-row position table")
 
 
 def init_run(args: AttrDict) -> None:
