@@ -39,7 +39,7 @@ typedef enum pmgt_status {
 } pmgt_status;
 
 /* ABI version of this header; bumped on any signature change. */
-#define PMGT_B200_ABI_VERSION 13
+#define PMGT_B200_ABI_VERSION 14
 int pmgt_abi_version(void);
 const char* pmgt_last_error(void);
 
@@ -322,6 +322,18 @@ typedef struct pmgt_attn_args {
 
 int pmgt_attn_core_fwd(const pmgt_attn_args* a, void* stream);
 int pmgt_attn_core_bwd(const pmgt_attn_args* a, void* stream);
+
+/*
+ * Attention maps: maps [rows][heads][L][L] fp32 receives, per (sequence, head),
+ * the matrix pmgt_attn_core_fwd multiplies V with for the same arguments,
+ *   A = beta * dropout(P1) + (1 - beta) * dropout(P2),
+ * with the very dropout mask the core applies for that shape, seed and site
+ * (ctx = A V).  Reads qkvc, mask, beta, dropout_*, rows, L, H and heads; ctx,
+ * dctx, dqkvc and d_bias_qkvc are ignored.  qkvc and maps must be 16-byte
+ * aligned; the shape limits are those of pmgt_attn_core_fwd.  Every check is
+ * made before any CUDA call.
+ */
+int pmgt_attn_maps_fwd(const pmgt_attn_args* a, float* maps, void* stream);
 
 /*
  * y = LayerNorm(dropout(o) + res) -- BertSelfOutput / BertOutput after their

@@ -11,7 +11,7 @@ import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libpmgt_b200.so")
-ABI_VERSION = 13
+ABI_VERSION = 14
 
 _lib = None
 
@@ -229,6 +229,7 @@ SIGNATURES = {
     "pmgt_embed_multi_bwd": (C.c_int, [C.POINTER(EmbedMultiArgs), c_vp]),
     "pmgt_attn_core_fwd": (C.c_int, [C.POINTER(AttnArgs), c_vp]),
     "pmgt_attn_core_bwd": (C.c_int, [C.POINTER(AttnArgs), c_vp]),
+    "pmgt_attn_maps_fwd": (C.c_int, [C.POINTER(AttnArgs), c_vp, c_vp]),
     "pmgt_res_ln_fwd": (C.c_int, [C.POINTER(ResLnArgs), c_vp]),
     "pmgt_res_ln_bwd": (C.c_int, [C.POINTER(ResLnArgs), c_vp]),
     "pmgt_linear_tile_supported": (C.c_int, [C.c_int64, C.c_int64, C.c_int, C.c_int]),

@@ -3,7 +3,8 @@
 // backward, over sequences of L = max_ctx_neigh + 1 tokens (6 by default).
 //
 // pmgt_attn_core_fwd / _bwd validate the arguments and pick one kernel family
-// from the shape alone (attn_family):
+// from the shape alone (attn_family); pmgt_attn_maps_fwd writes the attention
+// maps A (below) with the dropout mask of that family (attention_maps.cu):
 //   attn_mma  (attention_mma.cu)  L = 6,           head size 32 / 64 / 128
 //   attn_reg  (attention_reg.cu)  8 < L <= 64,     head size 32 / 64 / 128
 //   attn_mid  (attention_mid.cu)  8 < L <= 64,     other head sizes that are a multiple of 16, if its
@@ -318,6 +319,71 @@ static int attn_generic(const pmgt_attn_args* a, bool bwd, cudaStream_t st) {
   return PMGT_OK;
 }
 
+// Attention maps (pmgt_attn_maps_fwd) for head sizes that are not a multiple of 16: the forward kernel above up to A,
+// which goes to maps [rows][heads][L][L] fp32 instead of into A V.  Same arithmetic, same dropout stream.
+__global__ void __launch_bounds__(128) attn_maps_generic_kernel(const pmgt_attn_args a, float* __restrict__ maps,
+                                                                int warps_per_cta, AttnSmemLayout lay) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  if (wib >= warps_per_cta) return;
+  const int L = a.L, H = a.H, heads = a.heads, dh = H / heads, rs = lay.row_stride;
+  unsigned char* base = smem + (size_t)wib * lay.per_warp_fwd;
+  uint16_t* q = reinterpret_cast<uint16_t*>(base);
+  uint16_t* k = reinterpret_cast<uint16_t*>(base + lay.tile_bytes);
+  uint16_t* c = reinterpret_cast<uint16_t*>(base + 3 * lay.tile_bytes);
+  float* s1 = reinterpret_cast<float*>(base + 4 * lay.tile_bytes);
+  float* s2 = reinterpret_cast<float*>(base + 4 * lay.tile_bytes + lay.mat_bytes);
+  float* nrm = reinterpret_cast<float*>(base + 4 * lay.tile_bytes + 2 * lay.mat_bytes);
+  float* madd = nrm + ((L + 3) & ~3);
+  const long long n_items = a.rows * heads;
+  const long long w0 = (long long)blockIdx.x * warps_per_cta + wib;
+  const long long nw = (long long)gridDim.x * warps_per_cta;
+  const long long ld = 4ll * H;
+  const float keep_scale = a.dropout_p > 0.f ? 1.f / (1.f - a.dropout_p) : 1.f;
+  for (long long item = w0; item < n_items; item += nw) {
+    const long long row = item / heads;
+    const int head = (int)(item - row * heads);
+    const uint16_t* src = a.qkvc + row * L * ld + head * dh;
+    stage_rows(q, rs, src, ld, L, dh, lane);
+    stage_rows(k, rs, src + H, ld, L, dh, lane);
+    stage_rows(c, rs, src + 3 * H, ld, L, dh, lane);
+    __syncwarp();
+    scores_and_probs(q, k, c, rs, a.mask + row * L, L, dh, lane, s1, s2, nrm, madd, nullptr);
+    float* out = maps + item * L * L;
+    for (int e = lane; e < L * L; e += 32) {
+      float p1 = s1[e], p2 = s2[e];
+      if (a.dropout_p > 0.f) {
+        const uint64_t idx = (uint64_t)item * L * L + e;
+        p1 = dropout_keep(a.dropout_seed, a.dropout_site, idx, a.dropout_p) ? p1 * keep_scale : 0.f;
+        p2 = dropout_keep(a.dropout_seed, a.dropout_site + 1, idx, a.dropout_p) ? p2 * keep_scale : 0.f;
+      }
+      out[e] = a.beta * p1 + (1.f - a.beta) * p2;
+    }
+    __syncwarp();
+  }
+}
+
+static int attn_maps_generic(const pmgt_attn_args* a, float* maps, cudaStream_t st) {
+  const int dh = a->H / a->heads;
+  const AttnSmemLayout lay = attn_layout(a->L, dh);
+  const size_t per = lay.per_warp_fwd;
+  const size_t budget = 200 * 1024;
+  PMGT_REQUIRE(per <= budget, "attention: L=%d, head size %d needs %zu bytes of shared memory per warp (> %zu)", a->L, dh,
+               per, budget);
+  int warps = (int)(budget / per);
+  if (warps > 4) warps = 4;
+  const size_t smem = per * warps;
+  if (smem > 48 * 1024)
+    PMGT_CHECK_CUDA(cudaFuncSetAttribute(attn_maps_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const long long items = a->rows * a->heads;
+  long long ctas = (items + warps - 1) / warps;
+  const long long cap = (long long)num_sms() * 8;
+  if (ctas > cap) ctas = cap;
+  attn_maps_generic_kernel<<<(unsigned)ctas, 128, smem, st>>>(*a, maps, warps, lay);
+  PMGT_LAUNCH_CHECK();
+  return PMGT_OK;
+}
+
 // Launchers of the other kernel families; each assumes attn_family() chose it.
 int attn_mma_fwd(const pmgt_attn_args* a, cudaStream_t st);  // attention_mma.cu
 int attn_mma_bwd(const pmgt_attn_args* a, cudaStream_t st);
@@ -328,6 +394,7 @@ int attn_mid_bwd(const pmgt_attn_args* a, cudaStream_t st);
 bool attn_mid_fits(int L, int dh);
 int attn_long_fwd(const pmgt_attn_args* a, cudaStream_t st);  // attention_long.cu
 int attn_long_bwd(const pmgt_attn_args* a, cudaStream_t st);
+int attn_maps_mma(const pmgt_attn_args* a, float* maps, bool reg_stream, cudaStream_t st);  // attention_maps.cu
 
 enum class AttnFamily { Mma, Reg, Mid, Long, Generic };
 
@@ -349,16 +416,26 @@ static AttnFamily attn_family(const pmgt_attn_args* a) {
 
 static bool misaligned16(const void* p) { return ((uintptr_t)p & 15) != 0; }
 
-// the argument checks of both entry points, made before any CUDA call
-static int attn_check(const pmgt_attn_args* a, bool bwd) {
-  const char* fn = bwd ? "pmgt_attn_core_bwd" : "pmgt_attn_core_fwd";
-  PMGT_REQUIRE(a && a->qkvc && a->mask && (bwd ? a->dctx && a->dqkvc : a->ctx != nullptr), "%s: null argument", fn);
-  PMGT_REQUIRE(!misaligned16(a->qkvc), "%s: qkvc must be 16-byte aligned", fn);
-  if (bwd) {
-    PMGT_REQUIRE(!misaligned16(a->dctx), "%s: dctx must be 16-byte aligned", fn);
-    PMGT_REQUIRE(!misaligned16(a->dqkvc), "%s: dqkvc must be 16-byte aligned", fn);
+enum class AttnCall { Fwd, Bwd, Maps };
+
+// the argument checks of the entry points, made before any CUDA call (`maps`: pmgt_attn_maps_fwd's output)
+static int attn_check(const pmgt_attn_args* a, AttnCall call, const float* maps = nullptr) {
+  const bool bwd = call == AttnCall::Bwd;
+  if (call == AttnCall::Maps) {
+    const char* fn = "pmgt_attn_maps_fwd";
+    PMGT_REQUIRE(a && a->qkvc && a->mask && maps, "%s: null argument", fn);
+    PMGT_REQUIRE(!misaligned16(a->qkvc), "%s: qkvc must be 16-byte aligned", fn);
+    PMGT_REQUIRE(!misaligned16(maps), "%s: maps must be 16-byte aligned", fn);
   } else {
-    PMGT_REQUIRE(!misaligned16(a->ctx), "%s: ctx must be 16-byte aligned", fn);
+    const char* fn = bwd ? "pmgt_attn_core_bwd" : "pmgt_attn_core_fwd";
+    PMGT_REQUIRE(a && a->qkvc && a->mask && (bwd ? a->dctx && a->dqkvc : a->ctx != nullptr), "%s: null argument", fn);
+    PMGT_REQUIRE(!misaligned16(a->qkvc), "%s: qkvc must be 16-byte aligned", fn);
+    if (bwd) {
+      PMGT_REQUIRE(!misaligned16(a->dctx), "%s: dctx must be 16-byte aligned", fn);
+      PMGT_REQUIRE(!misaligned16(a->dqkvc), "%s: dqkvc must be 16-byte aligned", fn);
+    } else {
+      PMGT_REQUIRE(!misaligned16(a->ctx), "%s: ctx must be 16-byte aligned", fn);
+    }
   }
   PMGT_REQUIRE(a->heads >= 1 && a->H % a->heads == 0, "attention: H must be divisible by heads");
   PMGT_REQUIRE((a->H / a->heads) % 2 == 0, "attention: head size must be even");
@@ -373,7 +450,7 @@ using namespace pmgt;
 extern "C" {
 
 int pmgt_attn_core_fwd(const pmgt_attn_args* a, void* stream) {
-  const int rc = attn_check(a, false);
+  const int rc = attn_check(a, AttnCall::Fwd);
   if (rc || a->rows == 0) return rc;
   const cudaStream_t st = (cudaStream_t)stream;
   switch (attn_family(a)) {
@@ -386,7 +463,7 @@ int pmgt_attn_core_fwd(const pmgt_attn_args* a, void* stream) {
 }
 
 int pmgt_attn_core_bwd(const pmgt_attn_args* a, void* stream) {
-  int rc = attn_check(a, true);
+  int rc = attn_check(a, AttnCall::Bwd);
   if (rc || a->rows == 0) return rc;
   const cudaStream_t st = (cudaStream_t)stream;
   switch (attn_family(a)) {
@@ -398,6 +475,16 @@ int pmgt_attn_core_bwd(const pmgt_attn_args* a, void* stream) {
   }
   if (rc == PMGT_OK && a->d_bias_qkvc) rc = pmgt_colsum_bf16(a->dqkvc, a->rows * a->L, 4ll * a->H, 4ll * a->H, a->d_bias_qkvc, stream);
   return rc;
+}
+
+// The maps draw the dropout mask of the family pmgt_attn_core_fwd runs for this shape: attn_reg's own stream, or the
+// common.cuh element stream of every other family.
+int pmgt_attn_maps_fwd(const pmgt_attn_args* a, float* maps, void* stream) {
+  const int rc = attn_check(a, AttnCall::Maps, maps);
+  if (rc || a->rows == 0) return rc;
+  const cudaStream_t st = (cudaStream_t)stream;
+  if ((a->H / a->heads) % 16 == 0) return attn_maps_mma(a, maps, attn_family(a) == AttnFamily::Reg, st);
+  return attn_maps_generic(a, maps, st);
 }
 
 }  // extern "C"

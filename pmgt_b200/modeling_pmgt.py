@@ -452,6 +452,18 @@ class _EncoderPlan:
         self.pending_backward = False
 
 
+class _EncoderOutputs:
+    """What an encoder pass collects besides its final hidden state (``output_hidden_states`` /
+    ``output_attentions``): ``layers`` = the bf16 ``[T, H]`` inputs of layers 0 .. n-1 (the embedding output, then the
+    outputs of layers 1 .. n-1), ``maps`` = per layer the fp32 ``[map_rows, heads, L, L]`` matrices its attention core
+    multiplied V with, for the first ``map_rows`` sequences."""
+    __slots__ = ("hidden", "attentions", "map_rows", "layers", "maps")
+
+    def __init__(self, hidden: bool, attentions: bool, map_rows: int):
+        self.hidden, self.attentions, self.map_rows = hidden, attentions, map_rows
+        self.layers, self.maps = [], []
+
+
 class _EncoderRun:
     """Activations of one encoder pass kept for the backward pass."""
     __slots__ = ("R", "L", "T", "mask", "rows_idx", "src", "src_rows", "proj", "x0", "layers", "seed", "p_hid",
@@ -478,7 +490,7 @@ def _tile_path(H: int, I: int) -> bool:
 
 def _encode_forward(fp: FlatParams, pre: str, cfg: PMGTConfig, src: List[torch.Tensor], rows_idx, R: int, L: int,
                     mask: torch.Tensor, training: bool, seed: int, keep: bool, hold: Optional[list] = None,
-                    last_rows: Optional[torch.Tensor] = None):
+                    last_rows: Optional[torch.Tensor] = None, outs: Optional[_EncoderOutputs] = None):
     """PMGTModel.forward (modeling_pmgt.py:80-152) on ``R`` sequences of length ``L``.
 
     ``src``: per modality either the bf16 feature table (``rows_idx`` = flat int64
@@ -490,6 +502,10 @@ def _encode_forward(fp: FlatParams, pre: str, cfg: PMGTConfig, src: List[torch.T
     LayerNorm, FFN, LayerNorm -- and their whole backward) only on those rows; the result is then the compact
     ``[len(last_rows), H]`` matrix.  In pre-training that is ~30 % of the tokens (all positions of the target and the
     masked-target rows, position 0 of the pair rows).
+
+    ``outs`` (opt-in): collect the per-layer hidden states and attention maps there (see ``_EncoderOutputs``).  The maps
+    come from pmgt_attn_maps_fwd with each layer's own attention arguments (same seed and site), right after its
+    attention core, so they carry the dropout mask that core applied.
     """
     H, I, heads = cfg.hidden_size, cfg.intermediate_size, cfg.num_attention_heads
     T = R * L
@@ -528,6 +544,15 @@ def _encode_forward(fp: FlatParams, pre: str, cfg: PMGTConfig, src: List[torch.T
                               fp.f32(E + "LayerNorm.weight"), fp.f32(E + "LayerNorm.bias"), cfg.layer_norm_eps, p_hid, seed,
                               0, x_out=x, row_idx=(rows_idx if dense_tables else None))
     ops.embed_multi_fwd(ea)
+    if outs is not None and outs.hidden and cfg.num_hidden_layers > 0:  # with no layers, x is the final state
+        outs.layers.append(x)
+
+    def collect_maps(i, qkvc):  # right after layer i's attention core, with its arguments
+        if outs is not None and outs.attentions:
+            maps = torch.empty(outs.map_rows, heads, L, L, dtype=torch.float32, device=dev)
+            ops.attn_maps_fwd(ops.attn_args(outs.map_rows, L, H, heads, float(cfg.beta), qkvc, mask, p_att, seed,
+                                            10 * (i + 1)), maps)
+            outs.maps.append(maps)
 
     run = None
     if keep:
@@ -556,6 +581,7 @@ def _encode_forward(fp: FlatParams, pre: str, cfg: PMGTConfig, src: List[torch.T
                         bias=fp.f32(P + "attention.self.query.bias", 4), tag="lt_qkvc_fwd")
         ctx = new(T, H)
         ops.attn_core_fwd(ops.attn_args(R, L, H, heads, float(cfg.beta), qkvc, mask, p_att, seed, site, ctx=ctx))
+        collect_maps(i, qkvc)
         Tl, x_res = T, x
         if last and compact:  # the rest of the last layer only for the rows somebody reads
             Tl = Tc
@@ -578,6 +604,8 @@ def _encode_forward(fp: FlatParams, pre: str, cfg: PMGTConfig, src: List[torch.T
                         site=site + 4, out_f32=(hidden_f32 if last else None), tag="lt_res_ln_fwd")
         if keep:
             run.layers.append((x, qkvc, ctx, z1, a, h_pre, h, z2))
+        if outs is not None and outs.hidden and not last:
+            outs.layers.append(y)
         x = y
     for i in range(0 if tile else n_layers):
         P = f"{pre}encoder.layer.{i}."
@@ -586,6 +614,7 @@ def _encode_forward(fp: FlatParams, pre: str, cfg: PMGTConfig, src: List[torch.T
         ops.linear_fwd(x, fp.bf16(P + "attention.self.query.weight", 4), fp.f32(P + "attention.self.query.bias", 4), qkvc)
         ctx = new(T, H)
         ops.attn_core_fwd(ops.attn_args(R, L, H, heads, float(cfg.beta), qkvc, mask, p_att, seed, site, ctx=ctx))
+        collect_maps(i, qkvc)
         o1 = new(T, H)
         ops.linear_fwd(ctx, fp.bf16(P + "attention.output.dense.weight"), fp.f32(P + "attention.output.dense.bias"), o1)
         a = new(T, H)
@@ -605,6 +634,8 @@ def _encode_forward(fp: FlatParams, pre: str, cfg: PMGTConfig, src: List[torch.T
                                       y=y, y_f32=(hidden_f32 if last else None)))
         if keep:
             run.layers.append((x, qkvc, ctx, o1, a, h_pre, h, o2))
+        if outs is not None and outs.hidden and not last:
+            outs.layers.append(y)
         x = y
     if n_layers == 0:
         hidden_f32 = x.float()
@@ -612,9 +643,14 @@ def _encode_forward(fp: FlatParams, pre: str, cfg: PMGTConfig, src: List[torch.T
 
 
 def _encode_backward(fp: FlatParams, pre: str, cfg: PMGTConfig, run: _EncoderRun, d_hidden: torch.Tensor,
-                     arena: GradArena, pool: Optional[_BufPool] = None):
+                     arena: GradArena, pool: Optional[_BufPool] = None, d_layers: Optional[list] = None):
     """Reverse of ``_encode_forward``; parameter gradients are accumulated into ``arena``.  ``pool`` (launch plans)
-    recycles the per-layer temporaries instead of leaving that to torch's allocator."""
+    recycles the per-layer temporaries instead of leaving that to torch's allocator.
+
+    ``d_layers`` (optional): fp32 ``[T, H]`` gradients (or None) of the inputs of layers 0 .. n-1, i.e. of the
+    ``_EncoderOutputs.layers`` hidden states.  The gradient of layer k's input joins the backward pass where layer k-1's
+    output LayerNorm reads its incoming gradient (its fp32 addend, otherwise unused there); that of the embedding output
+    is added to the gradient the embedding backward reads."""
     H, I, heads = cfg.hidden_size, cfg.intermediate_size, cfg.num_attention_heads
     R, L, T = run.R, run.L, run.T
     dev = d_hidden.device
@@ -706,6 +742,8 @@ def _encode_backward(fp: FlatParams, pre: str, cfg: PMGTConfig, run: _EncoderRun
         done(dy, dy_b, dz2, do2, dh_pre, da, dctx, *((do1,) if do1 is not dz1 else ()),
              *(() if BATCH_DW_QKVC else (dqkvc,)))
         dy, dy_b = dx, dz1  # d x = dx (projection branch) + dz1 (residual branch): summed by the consumer
+        if d_layers is not None and i > 0:
+            dy_f32 = d_layers[i]  # a loss on the hidden state between layers i - 1 and i
     if deferred_dw:
         ops.dw_tile_batch(deferred_dw)
         done(*(d[0] for d in deferred_dw))
@@ -748,9 +786,17 @@ def _encode_backward(fp: FlatParams, pre: str, cfg: PMGTConfig, run: _EncoderRun
         dx = new(T, H)
         ops.linear_dx(dqkvc, fp.bf16(P + "attention.self.query.weight", 4), dx, addend=dz1)
         dy = dx
+        if d_layers is not None and i > 0:
+            dy_f32 = d_layers[i]  # a loss on the hidden state between layers i - 1 and i
     if dy is None:  # zero layers
         dy = dy_f32.to(BF16)
         dy_b = None
+    elif d_layers is not None and d_layers[0] is not None:  # a loss on the embedding output
+        if dy_b is None:
+            dy_b = new(T, H)
+            ops.cast_f32_bf16(d_layers[0], dy_b)
+        else:
+            dy_b = (dy_b.float() + d_layers[0].view(T, H)).to(BF16)
     if fp.after_layers_hook is not None:
         ops.host_hook(fp.after_layers_hook, arena)
     # ---- embeddings
@@ -784,25 +830,40 @@ def _encode_backward(fp: FlatParams, pre: str, cfg: PMGTConfig, run: _EncoderRun
 
 class _EncodeFn(torch.autograd.Function):
     """Autograd node for one batched encoder pass.  ``params`` are passed only so
-    that autograd routes their gradients; the data is read from ``fp``."""
+    that autograd routes their gradients; the data is read from ``fp``.
+
+    With ``outs`` (per-layer outputs requested) the pass is never planned, and the fp32 ``[T, H]`` copies of
+    ``outs.layers`` are further outputs of the node, so their gradients reach the backward pass."""
 
     @staticmethod
-    def forward(ctx, host, src, rows_idx, mask, R, L, training, seed, arena, keep, last_rows, *params):
+    def forward(ctx, host, src, rows_idx, mask, R, L, training, seed, arena, keep, last_rows, outs, *params):
         fp, pre, cfg = host._fp, host._fp_prefix, host.config
-        plan = host._plan_for(fp, src, rows_idx, R, L, training, keep, arena, last_rows)
+        plan = host._plan_for(fp, src, rows_idx, R, L, training, keep, arena, last_rows) if outs is None else None
         host._active_plan = plan
         if plan is not None:
             hidden, run = plan.forward(fp, pre, cfg, src, rows_idx, mask, training, seed, keep, last_rows), None
         else:
             hidden, run = _encode_forward(fp, pre, cfg, src, rows_idx, R, L, mask, training, seed, keep,
-                                          last_rows=last_rows)
+                                          last_rows=last_rows, outs=outs)
         ctx.host, ctx.run, ctx.arena, ctx.n_params, ctx.plan, ctx.keep = host, run, arena, len(params), plan, keep
-        return hidden
+        ctx.hidden_shape = hidden.shape
+        if outs is None or not outs.hidden:
+            return hidden
+        ctx.set_materialize_grads(False)  # an output nobody differentiates arrives as None, not as zeros
+        return (hidden,) + tuple(x.float() for x in outs.layers)
 
     @staticmethod
-    def backward(ctx, d_hidden):
+    def backward(ctx, d_hidden, *d_layers):
         host, run, arena, plan = ctx.host, ctx.run, ctx.arena, ctx.plan
         fp, pre, cfg = host._fp, host._fp_prefix, host.config
+        if d_layers:
+            if d_hidden is None:
+                d_hidden = torch.zeros(ctx.hidden_shape, dtype=torch.float32, device=arena.fp.flat.device)
+            d_layers = [None if d is None else d.to(torch.float32).contiguous() for d in d_layers]
+            if all(d is None for d in d_layers):
+                d_layers = None
+        else:
+            d_layers = None
         if plan is not None:
             if not ctx.keep or not plan.pending_backward:
                 raise PMGTError("encoder backward called but the launch plan holds no activations for it")
@@ -810,10 +871,25 @@ class _EncodeFn(torch.autograd.Function):
         else:
             if run is None:
                 raise PMGTError("encoder backward called but activations were not kept")
-            _encode_backward(fp, pre, cfg, run, d_hidden, arena)
+            _encode_backward(fp, pre, cfg, run, d_hidden, arena, d_layers=d_layers)
             ctx.run = None
         grads = tuple(arena.view(n) for n in host._encoder_param_names)
-        return (None,) * 11 + grads
+        return (None,) * 12 + grads
+
+
+class _AttentionMapFn(torch.autograd.Function):
+    """Identity on an attention map that puts it into the autograd graph of the encoder pass (``anchor``) only to
+    refuse a backward pass through it: its gradient would need a new input to the backward kernel of every attention
+    family.  Without this node such a gradient would silently be dropped."""
+
+    @staticmethod
+    def forward(ctx, maps, anchor):
+        return maps.view_as(maps)
+
+    @staticmethod
+    def backward(ctx, g, _g_anchor=None):
+        raise NotImplementedError("attention maps (output_attentions) are not differentiable; detach them before "
+                                  "using them in a loss")
 
 
 class PMGTPretrainedModel(nn.Module):
@@ -847,6 +923,18 @@ class PMGTPretrainedModel(nn.Module):
     @property
     def dtype(self):
         return torch.float32
+
+
+def resolve_output_flags(config, output_attentions, output_hidden_states):
+    """transformers' rule: an explicit argument wins, otherwise the config's flag (False by default)."""
+    oa = output_attentions if output_attentions is not None else getattr(config, "output_attentions", False)
+    oh = output_hidden_states if output_hidden_states is not None else getattr(config, "output_hidden_states", False)
+    return bool(oa), bool(oh)
+
+
+def output_tuple(hidden_states, attentions) -> tuple:
+    """The optional tail of a ``return_dict=False`` tuple: ``hidden_states``, then ``attentions``, each if requested."""
+    return tuple(t for t in (hidden_states, attentions) if t is not None)
 
 
 _seed_counter = [0]
@@ -916,11 +1004,20 @@ class PMGTModel(PMGTPretrainedModel):
             self.__dict__["_encoder_params_cache"] = ps
         return ps
 
-    def encode(self, src, rows_idx, mask, R, L, arena=None, refresh=True, last_rows=None):
+    def encode(self, src, rows_idx, mask, R, L, arena=None, refresh=True, last_rows=None, *,
+               output_hidden_states=False, output_attentions=False, output_rows=None):
         """``src``: one bf16 source per modality (feature tables gathered through ``rows_idx``, or dense ``[R * L, D]``
         matrices when ``rows_idx`` is None).  ``last_rows`` (sorted unique token indices): return only those rows of
         the final hidden state, as a ``[len(last_rows), H]`` matrix; on the token-tile path the last layer's
         post-attention half is then computed for those rows only (see ``_encode_forward``).
+
+        ``output_hidden_states`` / ``output_attentions``: return ``(hidden, hidden_states, attentions)`` instead, for
+        the first ``output_rows`` sequences (default all ``R``).  ``hidden_states`` is a tuple of
+        ``num_hidden_layers`` fp32 ``[output_rows, L, H]`` tensors, the embedding output and the outputs of layers
+        1 .. n-1 (bf16 activations widened to fp32; the last layer's output is ``hidden``), and is differentiable.
+        ``attentions`` is a tuple of ``num_hidden_layers`` fp32 ``[output_rows, heads, L, L]`` tensors, the matrices
+        each layer multiplied V with (with this pass's dropout mask); a backward pass through one raises
+        ``NotImplementedError``.  Either is None when not requested.  Such a call never uses a launch plan.
 
         Raises ``ValueError``, before any device work, for a context longer than the position table or than the
         attention core's limit (MAX_CONTEXT_LEN tokens)."""
@@ -940,23 +1037,53 @@ class PMGTModel(PMGTPretrainedModel):
         src = tuple(src)
         if len(src) != len(cfg.feat_hidden_sizes):
             raise PMGTError(f"encode: {len(src)} feature sources for {len(cfg.feat_hidden_sizes)} modalities")
+        want = bool(output_hidden_states or output_attentions)
+        n_out = R if output_rows is None else int(output_rows)
+        outs = _EncoderOutputs(bool(output_hidden_states), bool(output_attentions), n_out) if want else None
         out = _EncodeFn.apply(self, src, rows_idx, mask, R, L, self.training, seed, arena, keep,
-                              last_rows if in_kernel else None, *params)
+                              last_rows if in_kernel else None, outs, *params)
+        layers = ()
+        if isinstance(out, tuple):
+            out, *layers = out
         if last_rows is not None and not in_kernel:  # other widths: encode everything, then pick the rows
             self._active_plan = None  # the gradient of the picked rows does not line up with the plan's buffer
             out = out.reshape(R * L, -1).index_select(0, last_rows)
-        return out
+        if not want:
+            return out
+        hidden_states = tuple(h.view(R, L, -1)[:n_out] for h in layers) if output_hidden_states else None
+        attentions = None
+        if output_attentions:
+            attentions = tuple(_AttentionMapFn.apply(m, out) if out.requires_grad else m for m in outs.maps)
+        return out, hidden_states, attentions
 
     def forward(self, *input_feat_embeds, attention_mask=None, head_mask=None, output_attentions=None,
                 output_hidden_states=None, return_dict=None):
+        """modeling_pmgt.py:80-152.  ``output_hidden_states`` / ``output_attentions`` (default: the config's) follow
+        transformers:
+
+        * ``hidden_states``: ``num_hidden_layers + 1`` fp32 ``[R, L, H]`` tensors, the embedding output and the output
+          of every layer; the last is ``last_hidden_state`` itself.  The others are the bf16 activations the encoder
+          keeps, widened to fp32.  They are differentiable: a loss on entry k reaches the parameters through the
+          backward pass of the layers below it.
+        * ``attentions``: ``num_hidden_layers`` fp32 ``[R, heads, L, L]`` tensors.  Entry k is the matrix layer k
+          multiplies the values with, ``beta * dropout(P1) + (1 - beta) * dropout(P2)`` (P1 the cosine softmax of the
+          context projections, P2 the scaled dot-product softmax, both with the -10000 key mask): rows sum to 1 in
+          eval mode, and in training they carry the dropout mask this pass applied.  They are not differentiable; a
+          backward pass through one raises ``NotImplementedError``.  They take ``4 * heads * L^2`` bytes per sequence
+          and layer (335 MB for 1,024 sequences of 128 tokens and 5 layers).
+
+        With ``return_dict=False`` they are appended to the tuple, ``hidden_states`` first, only when requested.  A call
+        that requests either never uses a launch plan.  ``head_mask`` is not supported."""
         assert len(input_feat_embeds) == len(self.config.feat_hidden_sizes), \
             f"# of multi-modal features must be {len(self.config.feat_hidden_sizes)}"
         first = input_feat_embeds[0]
         assert all(first.size()[:-1] == f.size()[:-1] for f in input_feat_embeds[1:]), \
             "All features are same dim except last one"
-        if head_mask is not None or output_attentions or output_hidden_states:
-            raise NotImplementedError("head_mask / output_attentions / output_hidden_states are not produced by the "
-                                      "fused kernels (the reference's trainer never requests them)")
+        if head_mask is not None:
+            raise NotImplementedError("head_mask is not supported by the fused attention kernels (the reference's "
+                                      "trainer never passes one)")
+        output_attentions, output_hidden_states = resolve_output_flags(self.config, output_attentions,
+                                                                       output_hidden_states)
         if not first.is_cuda:
             raise PMGTError("PMGTModel.forward needs CUDA tensors: pmgt_b200 has no CPU fallback")
         R, L = first.shape[:2]
@@ -964,10 +1091,19 @@ class PMGTModel(PMGTPretrainedModel):
         if attention_mask is None:
             attention_mask = torch.ones(R, L, device=first.device)
         dense = [f.reshape(R * L, f.shape[-1]).to(BF16).contiguous() for f in input_feat_embeds]
-        seq = self.encode(dense, None, attention_mask, R, L)
+        hidden_states = attentions = None
+        if output_attentions or output_hidden_states:
+            seq, inner, attentions = self.encode(dense, None, attention_mask, R, L,
+                                                 output_hidden_states=output_hidden_states,
+                                                 output_attentions=output_attentions)
+            if output_hidden_states:
+                hidden_states = inner + (seq,)
+        else:
+            seq = self.encode(dense, None, attention_mask, R, L)
         if not return_dict:
-            return (seq, None)
-        return BaseModelOutputWithPooling(last_hidden_state=seq, pooler_output=None)
+            return (seq, None) + output_tuple(hidden_states, attentions)
+        return BaseModelOutputWithPooling(last_hidden_state=seq, pooler_output=None, hidden_states=hidden_states,
+                                          attentions=attentions)
 
 
 # ---------------------------------------------------------------------------

@@ -23,7 +23,8 @@ import torch.nn as nn
 from ._lib import PMGTError
 from .configuration_pmgt import PMGTConfig
 from .modeling_pmgt import (BF16, FlatParams, GradArena, PMGTForPreTrainingOutput, PMGTGraphConstructLoss, PMGTModel,
-                            PMGTNodeConstructLoss, PMGTPretrainedModel, encoder_param_order)
+                            PMGTNodeConstructLoss, PMGTPretrainedModel, encoder_param_order, output_tuple,
+                            resolve_output_flags)
 from .utils import get_input_feat_embeds  # noqa: F401  (re-exported like the reference module)
 
 
@@ -288,11 +289,18 @@ class PMGT(PMGTPretrainedModel):
         return_dict: Optional[bool] = None,
         masked_inputs=None,
     ):
+        """models.py:56-176.  ``output_hidden_states`` / ``output_attentions`` (default: the config's) describe the
+        encoding of the TARGET contexts only (the pass whose ``last_hidden_state`` is returned), not the pairs or the
+        masked targets: ``hidden_states`` = ``num_hidden_layers + 1`` fp32 ``[B, L, H]`` tensors ending with
+        ``last_hidden_state``, ``attentions`` = ``num_hidden_layers`` fp32 ``[B, heads, L, L]`` tensors, with the
+        semantics, gradients and memory cost documented at ``PMGTModel.forward``.  With ``return_dict=False`` they are
+        appended to the tuple, ``hidden_states`` first, only when requested."""
         if pair_node_inputs is not None:
             assert labels is not None, "labels must be passed, when set pair_node_inputs"
             assert num_pairs is not None, "num_pairs must be passed, when set pair_node_inputs"
-        if output_attentions or output_hidden_states:
-            raise NotImplementedError("attention maps / per-layer hidden states are not produced by the fused kernels")
+        output_attentions, output_hidden_states = resolve_output_flags(self.config, output_attentions,
+                                                                       output_hidden_states)
+        want = output_attentions or output_hidden_states
         return_dict = return_dict if return_dict is not None else self.config.use_return_dict
 
         t_ids = target_node_inputs["node_ids"]
@@ -305,7 +313,8 @@ class PMGT(PMGTPretrainedModel):
         tables = self.feature_tables_bf16()
         # launch plans need the gradients of every step at the same address; the persistent arena is only safe while
         # no gradient of an earlier step is still attached (zero_grad(set_to_none=True) between steps)
-        if (self.bert.use_launch_plans and torch.is_grad_enabled() and all(p.grad is None for p in fp.params)
+        # (a call that asks for per-layer outputs is never planned: it keeps the plans' arena out of it too)
+        if (self.bert.use_launch_plans and not want and torch.is_grad_enabled() and all(p.grad is None for p in fp.params)
                 and not any(pl.pending_backward for pl in self.bert._plans.values())):
             arena = fp.step_arena()
         else:
@@ -332,9 +341,15 @@ class PMGT(PMGTPretrainedModel):
             ids_flat, mask_all = t_ids.reshape(-1), t_mask
         ids_flat = ids_flat.contiguous()
         R = mask_all.shape[0]
+        # the targets are the first B sequences of the batched pass: per-layer outputs are taken for those only
+        extra = dict(output_hidden_states=output_hidden_states, output_attentions=output_attentions,
+                     output_rows=B) if want else {}
+        inner = attentions = None
         if pair_node_inputs is None:
             hidden = self.bert.encode(tables, ids_flat, mask_all, R, L,
-                                      arena=arena, refresh=False)  # (R, L, H) fp32
+                                      arena=arena, refresh=False, **extra)  # (R, L, H) fp32
+            if want:
+                hidden, inner, attentions = hidden
             H = hidden.shape[-1]
             last_hidden_state = hidden[:B]
         else:
@@ -344,9 +359,12 @@ class PMGT(PMGTPretrainedModel):
             dev = t_ids.device
             sel = self._last_rows(B, SP, L, nfr_on, dev)
             hidden = self.bert.encode(tables, ids_flat, mask_all, R, L,
-                                      arena=arena, refresh=False, last_rows=sel)  # (Tc, H) fp32
+                                      arena=arena, refresh=False, last_rows=sel, **extra)  # (Tc, H) fp32
+            if want:
+                hidden, inner, attentions = hidden
             H = hidden.shape[-1]
             last_hidden_state = hidden[:B * L].view(B, L, H)
+        hidden_states = inner + (last_hidden_state,) if output_hidden_states else None
 
         loss = None
         prediction_logits = None
@@ -365,6 +383,7 @@ class PMGT(PMGTPretrainedModel):
                 plan.grad_buffer() if plan is not None and hidden.requires_grad else None, *nfr_params)
 
         if not return_dict:
-            return (loss, prediction_logits, last_hidden_state, None)
+            return (loss, prediction_logits, last_hidden_state, None) + output_tuple(hidden_states, attentions)
         return PMGTForPreTrainingOutput(loss=loss, prediction_logits=prediction_logits,
-                                        last_hidden_state=last_hidden_state)
+                                        last_hidden_state=last_hidden_state, hidden_states=hidden_states,
+                                        attentions=attentions)

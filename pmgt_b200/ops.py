@@ -431,6 +431,13 @@ def attn_core_fwd(a: AttnArgs):
          6 * T * a.L * a.H)
 
 
+def attn_maps_fwd(a: AttnArgs, maps):
+    """The matrices ``attn_core_fwd(a)`` multiplies V with, as fp32 ``maps`` [rows, heads, L, L] (same dropout mask)."""
+    T = a.rows * a.L
+    _run("attn_maps_fwd", _lib.lib().pmgt_attn_maps_fwd, (C.byref(a), ptr(maps), cur_stream()), 1,
+         6 * T * a.H + 4 * T * a.heads * a.L, 4 * T * a.L * a.H)
+
+
 def attn_core_bwd(a: AttnArgs):
     T = a.rows * a.L
     n_col = (4 * a.H + 2047) // 2048 if a.d_bias_qkvc else 0
